@@ -349,6 +349,44 @@ int irt_xchg_status(irt_xchg *x); /* 0, or 1 + rank of a peer whose flag never a
  * sum(12*nb + 8) + 8*Nb^3 + ceil(n/8) */
 int64_t irt_check_sets_algorithmic_bytes(const irt_setstore *store, int64_t begin, int64_t end);
 
+/* ---- exact k-nearest neighbours: replaces the host scans behind nn_->nearestK / nnTip_->nearestK
+ * (KBoundedStrategy, VoxelCachedLazyPRM.cpp:1329-1345; roadmapIk .cpp:3095-3137; addMilestone .cpp:1854-1885) --
+ * A device-resident, append-only point set with one metric.  The metric is the distance of OMPL's compound space
+ * of Problem.cpp:118-141 as both host mirrors compute it, or plain R^n:
+ *
+ *   d(a,b) = ((e + w_so2*s) + w_lin*l)        a term whose column is -1 is left out (not added as zero)
+ *   e = sqrt(((0 + t_0) + t_1) + ... + t_{n_euclid-1}),  t_j = (a_j - b_j)*(a_j - b_j)
+ *   s = |a_c - b_c|, then 2*M_PI - s if s > M_PI          (c = so2_col, pi and 2 pi as doubles)
+ *   l = |a_l - b_l|                                       (l = lin_col)
+ *
+ * in IEEE double, every operation rounded on its own (no FMA contraction), sums left to right, sqrt correctly
+ * rounded: bit for bit what VoxelCachedLazyPRM::distance of host/irt_host.hpp computes.  The Euclidean columns are
+ * the leading n_euclid columns; so2_col / lin_col must lie after them and differ.  Weights are finite and >= 0.
+ * Other columns are stored but never read.
+ *
+ * irt_nnset_knn: for each of m query rows, the k nearest items in (distance, index) order -- exactly what a stable
+ * sort by distance gives, also on exact ties -- skipping items whose exclude bit is set and returning only finite
+ * distances <= bound (NaN distances never).  Entries past the last hit are idx -1 / dist +inf.  Host pointers,
+ * synchronous.  IRT_ERR_INVALID_ARGUMENT for k outside [1, IRT_KNN_MAX_K], dim outside [1, 16] or a bad metric;
+ * IRT_ERR_CAPACITY past 2^31 - 2 items.  n = 0 and m = 0 are valid. */
+typedef struct irt_metric {
+  int32_t n_euclid; /* leading columns under the L2 norm (tensions; 3 for tip positions) */
+  int32_t so2_col;  /* column of an SO(2) angle, -1 = none */
+  int32_t lin_col;  /* column under a weighted |difference| (retraction), -1 = none */
+  int32_t _pad;
+  double w_so2, w_lin;
+} irt_metric;
+#define IRT_KNN_MAX_K 64
+typedef struct irt_nnset irt_nnset;
+int irt_nnset_create(irt_ctx *ctx, int dim, const irt_metric *m, irt_nnset **out);
+void irt_nnset_destroy(irt_nnset *s);
+int64_t irt_nnset_size(const irt_nnset *s);
+int irt_nnset_append(irt_ctx *ctx, irt_nnset *s, const double *rows /* [n][dim] host */, int64_t n);
+int irt_nnset_clear(irt_ctx *ctx, irt_nnset *s);
+int irt_nnset_knn(irt_ctx *ctx, const irt_nnset *s, const double *queries /* [m][dim] */, int64_t m, int k,
+                  double bound, const uint32_t *exclude_words /* NULL, or bit i % 32 of word i / 32 */,
+                  int64_t *idx /* [m][k] */, double *dist /* [m][k] or NULL */);
+
 /* ---- .rmp roadmap files (SURVEY 8f "next" #1) ----------------------------------------------
  * The reference's binary roadmap format: LazyRmpParser / RmpStreamer
  * (motion-planning/VoxelCachedLazyPRM.cpp:862-1114, serialize_inner :636-657):

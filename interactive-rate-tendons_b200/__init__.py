@@ -10,6 +10,7 @@ sm_100a).  It mirrors the reference's operator interface for this path:
                        (motion-planning/VoxelCachedLazyPRM.h:141,165-179)
   Roadmap          <-> the batch entry points of VoxelCachedLazyPRM
                        (VoxelCachedLazyPRM.h:495-520; .cpp:1563-1782)
+  NearestSet       <-> the exact scans behind nn_ / nnTip_ (ompl::NearestNeighbors) of the planner
 
 There is no CPU fallback: if the CUDA library or a CUDA device is missing, construction fails
 loudly.  Nothing in this package imports the oracle/ directory.
@@ -83,6 +84,15 @@ class Rmp(C.Structure):
                 ("e_off", C.c_void_p), ("e_keys", C.c_void_p), ("e_bits", C.c_void_p)]
 
 
+class Metric(C.Structure):
+    """irt_metric: d = ((e + w_so2 s) + w_lin l), e = the L2 norm of the leading n_euclid columns (include/irt_b200.h)"""
+    _fields_ = [("n_euclid", C.c_int32), ("so2_col", C.c_int32), ("lin_col", C.c_int32), ("_pad", C.c_int32),
+                ("w_so2", C.c_double), ("w_lin", C.c_double)]
+
+
+KNN_MAX_K = 64
+
+
 class FkOutputs(C.Structure):
     _fields_ = [("p", C.c_void_p), ("R", C.c_void_p), ("t", C.c_void_p), ("npts", C.c_void_p),
                 ("L", C.c_void_p), ("L_i", C.c_void_p), ("tip", C.c_void_p), ("uv", C.c_void_p),
@@ -110,6 +120,8 @@ ABI_SYMBOLS = [
     "irt_xchg_create", "irt_xchg_destroy", "irt_xchg_handle_size", "irt_xchg_export", "irt_xchg_connect",
     "irt_check_sets_allgather_dev", "irt_xchg_status",
     "irt_rmp_read", "irt_rmp_write", "irt_rmp_free",
+    "irt_nnset_create", "irt_nnset_destroy", "irt_nnset_size", "irt_nnset_append", "irt_nnset_clear",
+    "irt_nnset_knn",
 ]
 
 _lib = None
@@ -188,6 +200,12 @@ def lib():
         "irt_rmp_read": (i32, [C.c_char_p, C.POINTER(C.POINTER(Rmp))]),
         "irt_rmp_write": (i32, [C.c_char_p, C.POINTER(Rmp)]),
         "irt_rmp_free": (None, [C.POINTER(Rmp)]),
+        "irt_nnset_create": (i32, [vp, i32, C.POINTER(Metric), C.POINTER(vp)]),
+        "irt_nnset_destroy": (None, [vp]),
+        "irt_nnset_size": (i64, [vp]),
+        "irt_nnset_append": (i32, [vp, vp, vp, i64]),
+        "irt_nnset_clear": (i32, [vp, vp]),
+        "irt_nnset_knn": (i32, [vp, vp, vp, i64, i32, C.c_double, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         f = getattr(L, name)
@@ -628,6 +646,86 @@ class SetStore:
     def algorithmic_bytes(self, begin=0, end=None):
         end = self.num_sets if end is None else end
         return int(self.ctx.L.irt_check_sets_algorithmic_bytes(self.h, begin, end))
+
+
+def state_metric(spec):
+    """irt_metric of the compound state space (Problem.cpp:118-141) with the weights computed exactly as
+    roadmap.VoxelCachedLazyPRM.distance computes them: tensions under L2, rotation weighted ext / (4 pi), retraction
+    weighted 2 ext / L, ext = |max_tension|.  Returns (state size, Metric)."""
+    N = len(spec["C"])
+    ext = float(np.linalg.norm(np.asarray(spec["max_tension"], dtype=np.float64)[:N]))
+    m = Metric(N, -1, -1, 0, 0.0, 0.0)
+    k = N
+    if spec.get("enable_rotation"):
+        m.so2_col, m.w_so2 = k, ext / (4 * np.pi)
+        k += 1
+    if spec.get("enable_retraction"):
+        m.lin_col, m.w_lin = k, 2 * ext / spec["L"]
+        k += 1
+    return k, m
+
+
+def tip_metric():
+    """plain R^3, as np.linalg.norm(tips - request, axis=1)"""
+    return Metric(3, -1, -1, 0, 0.0, 0.0)
+
+
+def pack_mask(flags):
+    """bool[n] -> the uint32 exclude words of NearestSet.knn (bit i % 32 of word i / 32)"""
+    b = np.packbits(np.asarray(flags, dtype=bool), bitorder="little")
+    w = np.zeros(-(-len(b) // 4) * 4, dtype=np.uint8)
+    w[:len(b)] = b
+    return w.view(np.uint32)
+
+
+class NearestSet:
+    """Device-resident, append-only point set with exact k-nearest-neighbour queries (irt_nnset_*): the answers are
+    the same indices in the same order as a stable sort of the distances of the contract in include/irt_b200.h."""
+
+    def __init__(self, ctx, dim, metric):
+        self.ctx, self.dim, self.metric = ctx, int(dim), metric
+        h = C.c_void_p()
+        ctx.check(ctx.L.irt_nnset_create(ctx.h, self.dim, C.byref(metric), C.byref(h)))
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None) and getattr(self.ctx, "h", None):
+            self.ctx.L.irt_nnset_destroy(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def size(self):
+        return int(self.ctx.L.irt_nnset_size(self.h))
+
+    def append(self, rows):
+        rows = _np(rows, np.float64).reshape(-1, self.dim)
+        if len(rows):
+            self.ctx.check(self.ctx.L.irt_nnset_append(self.ctx.h, self.h, _ptr(rows), len(rows)))
+
+    def clear(self):
+        self.ctx.check(self.ctx.L.irt_nnset_clear(self.ctx.h, self.h))
+
+    def knn(self, queries, k, bound=np.inf, exclude=None):
+        """queries [m][dim] -> (idx int64[m][k], dist float64[m][k]); missing entries are -1 / inf.  exclude: None,
+        bool[size()] or uint32 words (pack_mask)."""
+        q = _np(queries, np.float64).reshape(-1, self.dim)
+        m, k = len(q), int(k)
+        idx = np.empty((m, max(k, 0)), dtype=np.int64)
+        dist = np.empty((m, max(k, 0)))
+        words = None
+        if exclude is not None:
+            exclude = np.asarray(exclude)
+            words = pack_mask(exclude) if exclude.dtype == bool else _np(exclude, np.uint32)
+            if len(words) * 32 < self.size():
+                raise IrtError(IRT_ERR_INVALID_ARGUMENT, "exclude mask shorter than the set")
+        self.ctx.check(self.ctx.L.irt_nnset_knn(self.ctx.h, self.h, _ptr(q), m, k, float(bound), _ptr(words),
+                                                _ptr(idx), _ptr(dist)))
+        return idx, dist
 
 
 class _DeviceWords:

@@ -43,6 +43,10 @@
 #include <vector>
 
 #include "../../include/irt_b200.h"
+#ifdef IRT_TEST_OVER_STANDIN
+// built over the test-only stand-in of the C ABI (no GPU): irt_nnset_* come from a sequential host implementation
+#include "../../tests/cpp/knn_standin.hpp"
+#endif
 
 namespace irt {
 
@@ -1001,12 +1005,22 @@ public:
     irt::check(ctx_, irt_setstore_create(ctx_, &g, &estore_));
     irt::check(ctx_, irt_env_create(ctx_, &g, &env_));
     env_voxels_.upload_env(ctx_, env_);
+    // the exact k-NN scans on the device: states under the compound space's distance, tips under plain R^3
+    irt_metric sm{(int32_t)robot_.tendons.size(), -1, -1, 0, 0.0, 0.0};
+    int col = sm.n_euclid;
+    if (robot_.enable_rotation) { sm.so2_col = col++; sm.w_so2 = tensionExtent() / (4.0 * M_PI); }
+    if (robot_.enable_retraction) { sm.lin_col = col++; sm.w_lin = 2.0 * tensionExtent() / robot_.specs.L; }
+    const irt_metric tm{3, -1, -1, 0, 0.0, 0.0};
+    irt::check(ctx_, irt_nnset_create(ctx_, (int)robot_.state_size(), &sm, &nn_states_.set));
+    irt::check(ctx_, irt_nnset_create(ctx_, 3, &tm, &nn_tips_.set));
   }
   ~VoxelCachedLazyPRM() {
     irt_setstore_destroy(vstore_); irt_setstore_destroy(estore_); irt_env_destroy(env_);
+    irt_nnset_destroy(nn_states_.set); irt_nnset_destroy(nn_tips_.set);
   }
   void setRoadmap(std::vector<std::vector<double>> states, std::vector<std::pair<size_t, size_t>> edges) {
     states_ = std::move(states); edges_ = std::move(edges);
+    nn_states_.stale = true;
     vflags_.clear(); eflags_.clear();
     adj_edges_ = (size_t)-1; vertex_removed_.clear(); edge_removed_.clear();
     clearValidity();
@@ -1121,9 +1135,25 @@ public:
     std::set<std::pair<size_t, size_t>> have;
     for (auto &e : edges_) have.insert(std::minmax(e.first, e.second));
     std::vector<std::pair<size_t, size_t>> new_edges;
-    for (size_t v = Nv; v < N; v++)
-      for (size_t n : (connection_ ? connection_(v) : nearestKBounded(v)))
+    irt_nnset *nn = connection_ ? nullptr : nearestSet(false, k_);
+    std::vector<int64_t> nbr;
+    if (nn) {   // every new vertex's KBoundedStrategy neighbours in one device call
+      std::vector<double> q((N - Nv) * S);
+      for (size_t v = Nv; v < N; v++) std::copy(states_[v].begin(), states_[v].end(), q.begin() + (v - Nv) * S);
+      nbr.resize((N - Nv) * k_);
+      irt::check(ctx_, irt_nnset_knn(ctx_, nn, q.data(), (int64_t)(N - Nv), (int)k_, getRange(), nullptr, nbr.data(),
+                                     nullptr));
+    }
+    for (size_t v = Nv; v < N; v++) {
+      std::vector<size_t> cand;
+      if (nn) {
+        for (size_t j = 0; j < k_ && nbr[(v - Nv) * k_ + j] >= 0; j++) cand.push_back((size_t)nbr[(v - Nv) * k_ + j]);
+      } else {
+        cand = connection_ ? connection_(v) : nearestKBounded(v);
+      }
+      for (size_t n : cand)
         if (n != v && have.insert(std::minmax(v, n)).second) new_edges.emplace_back(v, n);  // connectVertices
+    }
 
     // ---- voxelise / validate the new edges and remove the invalid ones (.cpp:1505-1551) ----
     if (voxelize_edges && !new_edges.empty()) {
@@ -1163,6 +1193,7 @@ public:
     std::vector<double> flat(n * S);
     for (size_t i = 0; i < n; i++) std::copy(states_[i].begin(), states_[i].end(), flat.begin() + i * S);
     vflags_.assign(n, 0); tips_.assign(3 * n, 0.0);
+    nn_tips_.stale = true;
     irt::check(ctx_, irt_voxelize_vertices(ctx_, robot_.handle(), flat.data(), (int)S, (int64_t)n, vstore_,
                                            vflags_.data(), tips_.data()));
   }
@@ -1179,7 +1210,7 @@ public:
   }
   void precomputeVoxelCache() { precomputeVertexVoxelCache(); precomputeEdgeVoxelCache(); }
   /// clear*VoxelCache (.cpp:1814-1829): drop the cached sets; validity words stay, like the reference's
-  void clearVertexVoxelCache() { clear_store(vstore_); vflags_.clear(); tips_.clear(); }
+  void clearVertexVoxelCache() { clear_store(vstore_); vflags_.clear(); tips_.clear(); nn_tips_.stale = true; }
   void clearEdgeVoxelCache() { clear_store(estore_); eflags_.clear(); }
   void clearVoxelCache() { clearVertexVoxelCache(); clearEdgeVoxelCache(); }
   size_t vertexVoxelCacheSize() const { return (size_t)irt_setstore_num_sets(vstore_); }
@@ -1355,6 +1386,15 @@ public:
   std::vector<size_t> nearestTips(const collision::Point &request, size_t k) {
     if (tips_.size() != 3 * states_.size()) precomputeVertexVoxelCache();
     build_adjacency();
+    if (irt_nnset *nn = nearestSet(true, k)) {
+      const std::vector<uint32_t> words = maskWords(vertex_removed_);
+      std::vector<int64_t> idx(k);
+      irt::check(ctx_, irt_nnset_knn(ctx_, nn, request.data(), 1, (int)k, INFINITY, words.data(), idx.data(), nullptr));
+      std::vector<size_t> out;
+      for (int64_t i : idx)
+        if (i >= 0) out.push_back((size_t)i);
+      return out;
+    }
     std::vector<std::pair<double, size_t>> d;
     for (size_t v = 0; v < states_.size(); v++) {
       if (vertex_removed_[v]) continue;
@@ -1551,6 +1591,7 @@ public:
     auto keep_vertex = [&](size_t i) {   // the result's vertex stays in the roadmap with its caches
       if (own[i] >= 0) {
         for (int c = 0; c < 3; c++) tips_[3 * (size_t)own[i] + c] = tips[3 * i + c];
+        nn_tips_.stale = true;
         vertex_validity_[(size_t)own[i]] = VALIDITY_TRUE;
         return (size_t)own[i];
       }
@@ -1602,16 +1643,13 @@ public:
     long v = findState(best_pe->last_valid);
     if (v < 0) {
       // addMilestone(state, true): connected lazily to its connection-strategy neighbours (itself not yet in nn_)
-      std::vector<std::pair<double, size_t>> d;
-      for (size_t u = 0; u < states_.size(); u++)
-        if (!vertex_removed_[u]) d.emplace_back(distance(best_pe->last_valid, states_[u]), u);
-      const size_t kk = std::min(k_, d.size());
-      std::partial_sort(d.begin(), d.begin() + kk, d.end());
+      const std::vector<size_t> conn = connectionNeighbors(best_pe->last_valid);
       v = (long)appendVertex(best_pe->last_valid, &tips[3 * bi]);   // the reference caches the IK RESULT's tip here
-      for (size_t j = 0; j < kk && d[j].first <= getRange(); j++) appendEdge((size_t)v, d[j].second, VALIDITY_UNKNOWN);
+      for (size_t u : conn) appendEdge((size_t)v, u, VALIDITY_UNKNOWN);
       best->added_vertex = v;
     } else {
       for (int c = 0; c < 3; c++) tips_[3 * (size_t)v + c] = tips[3 * bi + c];
+      nn_tips_.stale = true;
       vertex_validity_[(size_t)v] = VALIDITY_TRUE;
     }
     if (s >= 0 && v != s) {
@@ -1645,16 +1683,11 @@ public:
     build_adjacency();
     const long have = findState(state);
     if (have >= 0) return {(size_t)have, false};
-    std::vector<std::pair<double, size_t>> d;
-    if (connect)
-      for (size_t u = 0; u < states_.size(); u++)
-        if (!vertex_removed_[u]) d.emplace_back(distance(state, states_[u]), u);
-    const size_t kk = std::min(k_, d.size());
-    std::partial_sort(d.begin(), d.begin() + kk, d.end());
+    const std::vector<size_t> conn = connect ? connectionNeighbors(state) : std::vector<size_t>();
     if (tips_.size() != 3 * states_.size()) precomputeVertexVoxelCache();
     const collision::Point tip = robot_.forward_kinematics(state).back();
     const size_t v = appendVertex(state, tip.data(), VALIDITY_UNKNOWN);
-    for (size_t j = 0; j < kk && d[j].first <= getRange(); j++) appendEdge(v, d[j].second, VALIDITY_UNKNOWN);
+    for (size_t u : conn) appendEdge(v, u, VALIDITY_UNKNOWN);
     return {v, true};
   }
   struct ChainedStep {
@@ -1720,6 +1753,24 @@ private:
   std::vector<long> ikNearest(const std::vector<double> &x, long own, size_t ik_neighbor, bool accurate,
                               const std::vector<char> &removed) const {
     if (!accurate) return {(long)ik_neighbor};
+    if (irt_nnset *nn = nearestSet(false, k_)) {
+      const std::vector<uint32_t> words = maskWords(removed);
+      std::vector<int64_t> idx(k_);
+      std::vector<double> dist(k_);
+      irt::check(ctx_, irt_nnset_knn(ctx_, nn, x.data(), 1, (int)k_, getRange(), words.data(), idx.data(), dist.data()));
+      std::vector<long> out;
+      size_t zeros = 0;
+      for (size_t j = 0; j < k_ && idx[j] >= 0; j++) {
+        out.push_back((long)idx[j]);
+        zeros += dist[j] <= 0.0;
+      }
+      if (own < 0 && 0.0 <= getRange()) {   // the temporary vertex: distance 0, after every item at distance 0
+        out.insert(out.begin() + (long)zeros, -1L);
+        if (out.size() > k_) out.pop_back();
+      }
+      if (std::find(out.begin(), out.end(), (long)ik_neighbor) == out.end()) out.push_back((long)ik_neighbor);
+      return out;
+    }
     std::vector<std::pair<double, size_t>> d;
     for (size_t u = 0; u < states_.size(); u++)
       if (!removed[u]) d.emplace_back(distance(x, states_[u]), u);
@@ -1831,6 +1882,59 @@ private:
     const uint64_t bits = 0;
     irt::check(ctx_, irt_setstore_import(ctx_, st, 0, &off, &key, &bits));
   }
+  /// a device copy of states_ or tips_ for the k-NN queries: `rows` of them are on the device; `stale` = the host
+  /// array was replaced or written in place since (rebuilt before the next query; appends are appended)
+  struct NnMirror { irt_nnset *set = nullptr; size_t rows = 0; bool stale = false; };
+  /// the device set mirroring tips_ (tips) or states_, brought up to date, or nullptr where the host scans answer
+  /// (k outside [1, IRT_KNN_MAX_K])
+  irt_nnset *nearestSet(bool tips, size_t k) const {
+    if (k < 1 || k > IRT_KNN_MAX_K) return nullptr;
+    NnMirror &m = tips ? nn_tips_ : nn_states_;
+    const size_t S = robot_.state_size(), rows = tips ? tips_.size() / 3 : states_.size();
+    if (m.stale || m.rows > rows) {
+      irt::check(ctx_, irt_nnset_clear(ctx_, m.set));
+      m.rows = 0;
+      m.stale = false;
+    }
+    if (rows > m.rows) {
+      std::vector<double> flat;
+      if (tips) {
+        flat.assign(tips_.begin() + 3 * m.rows, tips_.end());
+      } else {
+        flat.resize((rows - m.rows) * S);
+        for (size_t i = m.rows; i < rows; i++) std::copy(states_[i].begin(), states_[i].end(), flat.begin() + (i - m.rows) * S);
+      }
+      irt::check(ctx_, irt_nnset_append(ctx_, m.set, flat.data(), (int64_t)(rows - m.rows)));
+      m.rows = rows;
+    }
+    return m.set;
+  }
+  static std::vector<uint32_t> maskWords(const std::vector<char> &flags) {
+    std::vector<uint32_t> w(flags.size() / 32 + 1, 0);
+    for (size_t i = 0; i < flags.size(); i++)
+      if (flags[i]) w[i >> 5] |= 1u << (i & 31);
+    return w;
+  }
+  /// connectionStrategy_ of a state that is not in nn_ yet (addMilestone): the k nearest milestones within the range,
+  /// removed ones left out, nearest first
+  std::vector<size_t> connectionNeighbors(const std::vector<double> &x) {
+    std::vector<size_t> out;
+    if (irt_nnset *nn = nearestSet(false, k_)) {
+      const std::vector<uint32_t> words = maskWords(vertex_removed_);
+      std::vector<int64_t> idx(k_);
+      irt::check(ctx_, irt_nnset_knn(ctx_, nn, x.data(), 1, (int)k_, getRange(), words.data(), idx.data(), nullptr));
+      for (int64_t i : idx)
+        if (i >= 0) out.push_back((size_t)i);
+      return out;
+    }
+    std::vector<std::pair<double, size_t>> d;
+    for (size_t u = 0; u < states_.size(); u++)
+      if (!vertex_removed_[u]) d.emplace_back(distance(x, states_[u]), u);
+    const size_t kk = std::min(k_, d.size());
+    std::partial_sort(d.begin(), d.begin() + kk, d.end());
+    for (size_t j = 0; j < kk && d[j].first <= getRange(); j++) out.push_back(d[j].second);
+    return out;
+  }
   /// exact k nearest of v among all milestones (v included, like nn_->nearestK), cut at the range
   std::vector<size_t> nearestKBounded(size_t v) const {
     std::vector<std::pair<double, size_t>> d(states_.size());
@@ -1876,6 +1980,7 @@ private:
   std::mt19937 gen_{20220801u};
   size_t k_ = 5;
   double range_ = 0.0;
+  mutable NnMirror nn_states_, nn_tips_;   // mutable: ikNearest is const and brings them up to date
 };
 
 }  // namespace motion_planning

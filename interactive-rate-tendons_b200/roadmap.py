@@ -8,8 +8,10 @@ Mirrors the batch entry points of the reference planner (motion-planning/VoxelCa
   precomputeVertexValidity()       :1563-1598     precomputeEdgeValidity()     :1600-1647
   clearValidity()                  :1656-1663     clear{Vertex,Edge}VoxelCache() :1814-1829
 
-The graph search, nearest-neighbour structures, IK and file formats of the reference planner
-stay on the host and are not re-implemented here; the roadmap is (states, edge index pairs).
+The graph search, IK and file formats of the reference planner stay on the host and are not re-implemented here;
+the roadmap is (states, edge index pairs).  The exact nearest-neighbour scans of the planner (connection strategy,
+nnTip_, addMilestone) run on the device through NearestSet when the planner has a library Context and k is at most
+KNN_MAX_K; otherwise the host scans below answer them, with the same indices in the same order.
 
 Multi-GPU (one process per GPU): vertices and edges are sharded by contiguous index range
 (boundaries aligned to 64 so verdict words never straddle shards), every rank voxelises and
@@ -22,7 +24,8 @@ torch.distributed (NCCL) only publishes the IPC handles once.  The plain all_gat
 """
 import numpy as np
 
-from . import (INVALID_MASK, FLAG_PARTIAL, Env, SetStore, make_space, shard_range, unpack_verdicts)
+from . import (INVALID_MASK, FLAG_PARTIAL, KNN_MAX_K, Context, Env, NearestSet, SetStore, make_space, shard_range,
+               state_metric, tip_metric, unpack_verdicts)
 
 VALIDITY_UNKNOWN = 0  # VoxelCachedLazyPRM.h:598-601
 VALIDITY_TRUE = 1
@@ -73,6 +76,24 @@ def _validity_table(collides, invalid):
     np.bitwise_or(c, invalid.view(np.uint8), out=c)
     np.bitwise_xor(c, 1, out=c)
     return c
+
+
+def connection_edges(nbr, nv0, old_edges, n):
+    """the edges the connection loop of createRoadmap adds, vectorised: nbr[i] = the neighbours (-1 = none) of vertex
+    nv0 + i, nearest first.  Same pairs in the same order as the loop -- new vertex ascending, then neighbour rank;
+    self-pairs dropped; the first occurrence of an unordered pair kept; pairs among old_edges dropped."""
+    nbr = np.asarray(nbr, dtype=np.int64)
+    v = np.repeat(np.arange(nv0, nv0 + len(nbr), dtype=np.int64), nbr.shape[1] if nbr.ndim == 2 else 0)
+    u = nbr.reshape(-1)
+    keep = (u >= 0) & (u != v)
+    v, u = v[keep], u[keep]
+    key = np.minimum(v, u) * n + np.maximum(v, u)
+    _, first = np.unique(key, return_index=True)
+    if len(old_edges):
+        old = np.sort(np.asarray(old_edges, dtype=np.int64).reshape(-1, 2), axis=1)
+        first = first[~np.isin(key[first], old[:, 0] * n + old[:, 1])]
+    first.sort()
+    return np.stack([v[first], u[first]], axis=1).reshape(-1, 2)
 
 
 class LockstepFk:
@@ -185,6 +206,45 @@ class VoxelCachedLazyPRM:
         self._vertex_unchecked, self._edge_unchecked = set(), set()
         self.max_uncached = 4096     # more items than this without a cached set: the next sweep rebuilds the cache
         self._flag_tables = {}
+        # device copies of self.states / self.tips for the k-NN queries: [set, rows it holds, must be rebuilt]
+        self._nn = None
+        if isinstance(ctx, Context):
+            dim, metric = state_metric(robot.spec)
+            self._nn = {"states": [NearestSet(ctx, dim, metric), 0, False],
+                        "tips": [NearestSet(ctx, 3, tip_metric()), 0, False]}
+
+    def _nearest_set(self, name, k):
+        """the NearestSet mirroring self.<name> ("states" / "tips"), brought up to date -- rows appended since the last
+        query are appended, a replaced or overwritten array is uploaded again -- or None where the host scans answer
+        (no library context, or k > KNN_MAX_K)"""
+        if self._nn is None or k > KNN_MAX_K:
+            return None
+        ent = self._nn[name]
+        rows = getattr(self, name)
+        rows = np.zeros((0, ent[0].dim)) if rows is None else rows
+        if ent[2] or ent[1] > len(rows):
+            ent[0].clear()
+            ent[1], ent[2] = 0, False
+        if len(rows) > ent[1]:
+            ent[0].append(rows[ent[1]:])
+            ent[1] = len(rows)
+        return ent[0]
+
+    def _replaced(self, name):
+        """self.<name> was replaced or written in place: its device copy is rebuilt before the next query"""
+        if self._nn is not None:
+            self._nn[name][2] = True
+
+    def _connection_neighbors(self, x, removed):
+        """connectionStrategy_ of a state x that is not in nn_ (addMilestone): the k nearest milestones within the
+        range, `removed` ones left out, on the device; None where the host scan answers"""
+        k = self.max_nearest_neighbors
+        nn = self._nearest_set("states", k)
+        if nn is None:
+            return None
+        idx, _ = nn.knn(np.asarray(x, dtype=np.float64)[None], k, self.range or 0.2 * self.maximum_extent(),
+                        exclude=removed)
+        return [int(j) for j in idx[0] if j >= 0]
 
     def _exchange(self, store, slot_words):
         """one exchange buffer per (store, slot size); creating it is collective (IPC handle all-gather)"""
@@ -197,6 +257,7 @@ class VoxelCachedLazyPRM:
     # ---- roadmap content ----------------------------------------------------------------
     def set_roadmap(self, states, edges):
         self.states = np.ascontiguousarray(states, dtype=np.float64)
+        self._replaced("states")
         self.edges = np.ascontiguousarray(edges, dtype=np.int64).reshape(-1, 2)
         self._have_vcache = self._have_ecache = False
         self._adj = None
@@ -316,6 +377,11 @@ class VoxelCachedLazyPRM:
                 have = set(map(tuple, np.sort(self.edges, axis=1).tolist()))
                 new_edges = np.array([e for e in new_edges.tolist() if tuple(sorted(e)) not in have],
                                      dtype=np.int64).reshape(-1, 2)
+        elif self._nearest_set("states", self.max_nearest_neighbors) is not None:
+            bound = self.range or 0.2 * self.maximum_extent()
+            nbr, _ = self._nearest_set("states", self.max_nearest_neighbors).knn(
+                self.states[nv0:n_vertices], self.max_nearest_neighbors, bound)
+            new_edges = connection_edges(nbr, nv0, self.edges, n_vertices)
         else:
             have = set(map(tuple, np.sort(self.edges, axis=1).tolist()))
             out = []
@@ -367,6 +433,7 @@ class VoxelCachedLazyPRM:
     def precomputeVertexVoxelCache(self):
         lo, hi = self.shard(len(self.states))
         self.vertex_flags, self.tips = self.vertex_store.voxelize_vertices(self.robot, self.states[lo:hi])
+        self._replaced("tips")
         self._have_vcache = True
         return self.vertex_flags
 
@@ -387,6 +454,7 @@ class VoxelCachedLazyPRM:
         """clearVertexVoxelCache (VoxelCachedLazyPRM.cpp:1814-1818): the cached sets go, validity words stay"""
         self.vertex_store = SetStore(self.ctx, self.grid)
         self.vertex_flags = self.tips = None
+        self._replaced("tips")
         self._have_vcache = False
         self._xchg = {k: v for k, v in self._xchg.items() if k[0] == id(self.edge_store)}
 
@@ -659,6 +727,11 @@ class VoxelCachedLazyPRM:
         """nnTip_->nearestK: the k vertices whose cached tip positions are nearest to `request` (exact)"""
         if self.tips is None or len(self.tips) != len(self.states):
             self.precomputeVertexVoxelCache()
+        nn = self._nearest_set("tips", k)
+        if nn is not None:
+            removed = self.vertex_removed if len(self.vertex_removed) == len(self.tips) else None
+            idx, _ = nn.knn(np.asarray(request, dtype=np.float64)[None], k, exclude=removed)
+            return idx[0][idx[0] >= 0]
         d = np.linalg.norm(self.tips - np.asarray(request, dtype=np.float64)[None], axis=1)
         d = np.where(self.vertex_removed[:len(d)] if len(self.vertex_removed) == len(d) else False, np.inf, d)
         order = np.lexsort((np.arange(len(d)), d))[:k]
@@ -705,6 +778,17 @@ class VoxelCachedLazyPRM:
         if not accurate:
             return [int(ik_neighbor)]
         bound = self.range or 0.2 * self.maximum_extent()
+        nn = self._nearest_set("states", self.max_nearest_neighbors)
+        if nn is not None:
+            idx, dist = nn.knn(np.asarray(x, dtype=np.float64)[None], self.max_nearest_neighbors, bound, exclude=removed)
+            hit = idx[0] >= 0
+            out = [int(j) for j in idx[0][hit]]
+            if own < 0 and 0.0 <= bound:  # the temporary vertex: distance 0, after every item at distance 0
+                out.insert(int((dist[0][hit] <= 0.0).sum()), -1)
+                out = out[:self.max_nearest_neighbors]
+            if int(ik_neighbor) not in out:
+                out.append(int(ik_neighbor))
+            return out
         d = self.distance(x, self.states)
         d = np.where(removed, np.inf, d)
         ids = np.arange(len(d))
@@ -770,6 +854,8 @@ class VoxelCachedLazyPRM:
             return v, False
         conn = []
         if connect and len(self.states):
+            conn = self._connection_neighbors(x, self.vertex_removed)
+        if conn is None:
             d = np.where(self.vertex_removed, np.inf, self.distance(x, self.states))
             order = np.lexsort((np.arange(len(d)), d))[:self.max_nearest_neighbors]
             conn = [int(j) for j in order if d[j] <= (self.range or 0.2 * self.maximum_extent())]
@@ -952,6 +1038,7 @@ class VoxelCachedLazyPRM:
                         v = self._append_vertex(bounded[i], tips[i])
                     else:
                         self.tips[v] = tips[i]
+                        self._replaced("tips")
                         self.vertex_validity[v] = VALIDITY_TRUE
                     return result(i, added_vertex=v if own[i] < 0 else None, already_in_roadmap=own[i] >= 0)
                 nearest[i].append(s)
@@ -961,6 +1048,7 @@ class VoxelCachedLazyPRM:
                         v = self._append_vertex(bounded[i], tips[i])
                     else:
                         self.tips[v] = tips[i]
+                        self._replaced("tips")
                         self.vertex_validity[v] = VALIDITY_TRUE
                     self._append_edges([[int(s), v]], VALIDITY_TRUE)
                     return result(i, added_vertex=v if own[i] < 0 else None, source=int(s))
@@ -983,14 +1071,17 @@ class VoxelCachedLazyPRM:
         added = v < 0
         if added:
             # addMilestone(state, true): connected lazily to its connection-strategy neighbours (itself not yet in nn_)
-            d = np.where(self.vertex_removed, np.inf, self.distance(e["last_valid"], self.states))
-            order = np.lexsort((np.arange(len(d)), d))[:self.max_nearest_neighbors]
-            conn = [int(j) for j in order if d[j] <= (self.range or 0.2 * self.maximum_extent())]
+            conn = self._connection_neighbors(e["last_valid"], self.vertex_removed)
+            if conn is None:
+                d = np.where(self.vertex_removed, np.inf, self.distance(e["last_valid"], self.states))
+                order = np.lexsort((np.arange(len(d)), d))[:self.max_nearest_neighbors]
+                conn = [int(j) for j in order if d[j] <= (self.range or 0.2 * self.maximum_extent())]
             v = self._append_vertex(e["last_valid"], tips[i])      # the reference caches the IK RESULT's tip here
             if conn:
                 self._append_edges([[v, n] for n in conn], VALIDITY_UNKNOWN)
         else:
             self.tips[v] = tips[i]
+            self._replaced("tips")
             self.vertex_validity[v] = VALIDITY_TRUE
         if s >= 0 and v != s:
             eid = self.edge_index(int(s), v)
