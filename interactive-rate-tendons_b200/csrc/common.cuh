@@ -38,7 +38,6 @@ struct irt_ctx {
   void *pinned = nullptr;
   size_t pinned_bytes = 0;
   bool debug_sync = false;   // IRT_B200_DEBUG_SYNC=1
-  bool fk_smem = false;      // IRT_FK_SMEM=1: K1 variant with the integration state in shared memory (if built)
 };
 
 // device-resident robot constants (passed to kernels by value)

@@ -110,8 +110,6 @@ int irt_ctx_create(int device, irt_ctx **out) {
   {
     const char *dbg = getenv("IRT_B200_DEBUG_SYNC");
     ctx->debug_sync = dbg && dbg[0] == '1';
-    const char *fs = getenv("IRT_FK_SMEM");
-    ctx->fk_smem = fs && fs[0] == '1';
   }
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) ctx->sm_count = prop.multiProcessorCount;

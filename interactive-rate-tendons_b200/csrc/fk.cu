@@ -28,27 +28,9 @@
 
 namespace {
 
-#ifndef FK_THREADS_PER_BLOCK
-#define FK_THREADS_PER_BLOCK 128
-#endif
-#ifndef FK_MIN_BLOCKS
-#define FK_MIN_BLOCKS 2
-#endif
-constexpr int FK_THREADS = FK_THREADS_PER_BLOCK;
+constexpr int FK_THREADS = 128;
+constexpr int FK_BLOCKS_PER_SM = 2;
 
-#ifndef FK_FAST_PRIMS
-#define FK_FAST_PRIMS 1
-#endif
-#ifndef FK_PERSIST
-#define FK_PERSIST 1
-#endif
-#ifndef FK_PIPELINE_TENDONS
-#define FK_PIPELINE_TENDONS 0
-#endif
-#ifndef FK_SMEM_VARIANT
-#define FK_SMEM_VARIANT 0
-#endif
-#if FK_FAST_PRIMS
 // Branch-free reciprocal / reciprocal square root: the hardware FP64 seed (MUFU.RCP64H /
 // MUFU.RSQ64H, ~20 bits) refined by two Newton steps (relative error ~1e-16, not correctly
 // rounded).  Unlike the library routines they contain no special-case branches, so the compiler
@@ -71,10 +53,6 @@ __device__ __forceinline__ double rsqrt_fast(double x) {
   e = fma(-hx * y, y, 0.5);
   return fma(y, e, y);
 }
-#else
-__device__ __forceinline__ double rcp_fast(double x) { return 1.0 / x; }
-__device__ __forceinline__ double rsqrt_fast(double x) { return rsqrt(x); }
-#endif
 
 // routing at arbitrary t, per thread (only used inside the irregular first gap); same
 // power-sum form as get_poly_vecs / get_r_info2 (tendon/get_r_info.cpp:17-40,105-144), with the
@@ -176,9 +154,6 @@ __device__ __forceinline__ void routing_eval_simple(const RobotDev &rb, const do
 // a DFMA with three distinct register pairs costs 3 issue cycles instead of 2 (irt_measure_fp64_rate mode 2:
 // 0.68 of the DFMA peak), and every routing value that comes from a uniform register is one pair less -- and the 36
 // values of a row no longer occupy 72 registers of every thread.
-#ifndef FK_CONST_TABLE
-#define FK_CONST_TABLE 1
-#endif
 constexpr int FK_CT_DOUBLES = 7680;   // 60 KB of the 64 KB constant bank: 213 rows of a 6-tendon robot
 __constant__ double c_fk_tab[FK_CT_DOUBLES];
 struct RtPtr {
@@ -205,43 +180,17 @@ __device__ __forceinline__ void vu_dot(const RT &rt, const double (&tau)[NT],
   // value of a sum can differ from the +0.0 start only in the sign of an exact zero
   double av0 = -0.0, av1 = -0.0, av2 = -0.0, bv0 = 0, bv1 = 0, bv2 = -0.0;
   double esum = -0.0, erx = -0.0, ery = -0.0, exx = 0, eyy = 0, exy = 0;
-#if FK_PIPELINE_TENDONS
-  // software pipeline over the tendons: the latency chain of tendon j+1 (q -> |q|^2 -> rsqrt seed -> two Newton
-  // steps, ~12 dependent FP64 operations) is started BEFORE the ~70 independent accumulations of tendon j, so the
-  // two overlap inside one warp (with 2 warps per scheduler there is nobody else to hide it)
-  double nqx, nqy, nqz, ns2, nrs;
-  {
-    const double rx = rt[0], ry = rt[1], dx = rt[2], dy = rt[3];
-    nqx = fma(-u[2], ry, dx + v[0]);
-    nqy = fma(u[2], rx, dy + v[1]);
-    nqz = fma(u[0], ry, fma(-u[1], rx, v[2]));
-    ns2 = fma(nqx, nqx, fma(nqy, nqy, nqz * nqz));
-    nrs = rsqrt_fast(ns2);
-  }
-#endif
 #pragma unroll
   for (int j = 0; j < NT; j++) {
     const double rx = rt[6 * j + 0], ry = rt[6 * j + 1];
     const double dx = rt[6 * j + 2], dy = rt[6 * j + 3];
     const double ddx = rt[6 * j + 4], ddy = rt[6 * j + 5];
-#if FK_PIPELINE_TENDONS
-    const double qx = nqx, qy = nqy, qz = nqz, s2 = ns2, rs = nrs;
-    if (j + 1 < NT) {
-      const double rx1 = rt[6 * j + 6], ry1 = rt[6 * j + 7], dx1 = rt[6 * j + 8], dy1 = rt[6 * j + 9];
-      nqx = fma(-u[2], ry1, dx1 + v[0]);
-      nqy = fma(u[2], rx1, dy1 + v[1]);
-      nqz = fma(u[0], ry1, fma(-u[1], rx1, v[2]));
-      ns2 = fma(nqx, nqx, fma(nqy, nqy, nqz * nqz));
-      nrs = rsqrt_fast(ns2);
-    }
-#else
     // q = u x r + r' + v        (r_z = r'_z = r''_z = 0)
     const double qx = fma(-u[2], ry, dx + v[0]);
     const double qy = fma(u[2], rx, dy + v[1]);
     const double qz = fma(u[0], ry, fma(-u[1], rx, v[2]));
     const double s2 = fma(qx, qx, fma(qy, qy, qz * qz));
     const double rs = rsqrt_fast(s2);
-#endif
     sig[j] = s2 * rs;
     const double e = tau[j] * rs;        // tau / sigma
     const double c3 = e * (rs * rs);     // tau / sigma^3
@@ -333,63 +282,21 @@ __device__ __forceinline__ void vu_dot(const RT &rt, const double (&tau)[NT],
   vd[2] = fma(-idA, fma(y20, ud[0], fma(y21, ud[1], y22 * ud[2])), z2);
 }
 
-// Integration state of one configuration.  SM = false: registers (255 per thread, 8 warps per SM).
-// SM = true: per-thread slots in shared memory with stride SM_THREADS (conflict-free): the state proper AND the
-// RK4 stage scratch live there, so that the derivative evaluation -- the only register-hungry part -- runs at
-// 168 registers and 12 warps per SM (3 per scheduler instead of 2) hide each other's FP64 latencies.
-#ifndef FK_SM_THREADS_PER_BLOCK
-#define FK_SM_THREADS_PER_BLOCK 384
-#endif
-#ifndef FK_SM_MIN_BLOCKS
-#define FK_SM_MIN_BLOCKS 1
-#endif
-constexpr int FK_SM_THREADS = FK_SM_THREADS_PER_BLOCK;
+// Integration state of one configuration; it lives in registers (255 per thread, 8 warps per SM).
 template <int NT>
-constexpr int fk_sm_slots() { return 19 + NT + 9 + 9 + 3 + 3; }   // R v u p L Li | sR aR av au
-
-template <int NT, bool SM>
-struct FkState;
-template <int NT>
-struct FkState<NT, false> {
-  double R_[9];  // column-major (R[i + 3 j]) like Eigen
-  double v_[3], u_[3];
-  double p_[3];
-  double Lb_;
-  double Li_[NT];
-  __device__ __forceinline__ double &R(int i) { return R_[i]; }
-  __device__ __forceinline__ const double &R(int i) const { return R_[i]; }
-  __device__ __forceinline__ double &V(int i) { return v_[i]; }
-  __device__ __forceinline__ const double &V(int i) const { return v_[i]; }
-  __device__ __forceinline__ double &U(int i) { return u_[i]; }
-  __device__ __forceinline__ const double &U(int i) const { return u_[i]; }
-  __device__ __forceinline__ double &P(int i) { return p_[i]; }
-  __device__ __forceinline__ const double &P(int i) const { return p_[i]; }
-  __device__ __forceinline__ double &LB() { return Lb_; }
-  __device__ __forceinline__ const double &LB() const { return Lb_; }
-  __device__ __forceinline__ double &LI(int j) { return Li_[j]; }
-  __device__ __forceinline__ const double &LI(int j) const { return Li_[j]; }
-};
-template <int NT>
-struct FkState<NT, true> {
-  double *sm;   // this thread's slot 0
-  __device__ __forceinline__ double &S(int slot) const { return sm[slot * FK_SM_THREADS]; }
-  __device__ __forceinline__ double &R(int i) const { return S(i); }
-  __device__ __forceinline__ double &V(int i) const { return S(9 + i); }
-  __device__ __forceinline__ double &U(int i) const { return S(12 + i); }
-  __device__ __forceinline__ double &P(int i) const { return S(15 + i); }
-  __device__ __forceinline__ double &LB() const { return S(18); }
-  __device__ __forceinline__ double &LI(int j) const { return S(19 + j); }
-  __device__ __forceinline__ double &SR(int i) const { return S(19 + NT + i); }
-  __device__ __forceinline__ double &AR(int i) const { return S(28 + NT + i); }
-  __device__ __forceinline__ double &AV(int i) const { return S(37 + NT + i); }
-  __device__ __forceinline__ double &AU(int i) const { return S(40 + NT + i); }
+struct FkState {
+  double R[9];  // column-major (R[i + 3 j]) like Eigen
+  double v[3], u[3];
+  double p[3];
+  double L;       // backbone length
+  double Li[NT];  // tendon lengths
 };
 
 // one classic RK4 step of size h; rt0/rt1/rt2 = routing at t, t+h/2, t+h.
 // The four stages are a real loop (not unrolled): the hot loop body is ONE copy of vu_dot, which
 // keeps the instruction footprint inside the SM's instruction cache.
 template <int NT, typename RT>
-__device__ __forceinline__ void rk4_step(FkState<NT, false> &x, const double (&tau)[NT],
+__device__ __forceinline__ void rk4_step(FkState<NT> &x, const double (&tau)[NT],
                                          const double (&Kse)[3], const double (&Kbt)[3], double h,
                                          const RT &rt0, const RT &rt1, const RT &rt2) {
   const double hh = 0.5 * h, w1 = h * (1.0 / 6.0), w2 = h * (1.0 / 3.0);
@@ -397,9 +304,9 @@ __device__ __forceinline__ void rk4_step(FkState<NT, false> &x, const double (&t
   double aR[9], av[3], au[3];      // k1 + 2 k2 + 2 k3 + k4
   double vd[3], ud[3], sig[NT], Rd[9];
 #pragma unroll
-  for (int i = 0; i < 3; i++) { sv[i] = x.V(i); su[i] = x.U(i); av[i] = 0.0; au[i] = 0.0; }
+  for (int i = 0; i < 3; i++) { sv[i] = x.v[i]; su[i] = x.u[i]; av[i] = 0.0; au[i] = 0.0; }
 #pragma unroll
-  for (int i = 0; i < 9; i++) { sR[i] = x.R(i); aR[i] = 0.0; }
+  for (int i = 0; i < 9; i++) { sR[i] = x.R[i]; aR[i] = 0.0; }
 
 #pragma unroll 1
   for (int stage = 0; stage < 4; stage++) {
@@ -412,17 +319,13 @@ __device__ __forceinline__ void rk4_step(FkState<NT, false> &x, const double (&t
     // p' = R v ; L' = |v| ; L_i' = sigma_i : pure quadratures, accumulate in place
 #pragma unroll
     for (int i = 0; i < 3; i++)
-      x.P(i) = fma(wq, fma(sR[i], sv[0], fma(sR[i + 3], sv[1], sR[i + 6] * sv[2])), x.P(i));
+      x.p[i] = fma(wq, fma(sR[i], sv[0], fma(sR[i + 3], sv[1], sR[i + 6] * sv[2])), x.p[i]);
     {
       const double vv = fma(sv[0], sv[0], fma(sv[1], sv[1], sv[2] * sv[2]));
-#if FK_FAST_PRIMS
-      x.LB() = fma(wq, vv * rsqrt_fast(vv), x.LB());
-#else
-      x.LB() = fma(wq, sqrt(vv), x.LB());
-#endif
+      x.L = fma(wq, vv * rsqrt_fast(vv), x.L);
     }
 #pragma unroll
-    for (int j = 0; j < NT; j++) x.LI(j) = fma(wq, sig[j], x.LI(j));
+    for (int j = 0; j < NT; j++) x.Li[j] = fma(wq, sig[j], x.Li[j]);
     // R' = R u^
 #pragma unroll
     for (int i = 0; i < 3; i++) {
@@ -431,79 +334,17 @@ __device__ __forceinline__ void rk4_step(FkState<NT, false> &x, const double (&t
       Rd[i + 6] = fma(sR[i], su[1], -sR[i + 3] * su[0]);
     }
 #pragma unroll
-    for (int i = 0; i < 9; i++) { aR[i] = fma(wk, Rd[i], aR[i]); sR[i] = fma(a, Rd[i], x.R(i)); }
+    for (int i = 0; i < 9; i++) { aR[i] = fma(wk, Rd[i], aR[i]); sR[i] = fma(a, Rd[i], x.R[i]); }
 #pragma unroll
     for (int i = 0; i < 3; i++) {
       av[i] = fma(wk, vd[i], av[i]); au[i] = fma(wk, ud[i], au[i]);
-      sv[i] = fma(a, vd[i], x.V(i)); su[i] = fma(a, ud[i], x.U(i));
+      sv[i] = fma(a, vd[i], x.v[i]); su[i] = fma(a, ud[i], x.u[i]);
     }
   }
 #pragma unroll
-  for (int i = 0; i < 9; i++) x.R(i) = fma(w1, aR[i], x.R(i));
+  for (int i = 0; i < 9; i++) x.R[i] = fma(w1, aR[i], x.R[i]);
 #pragma unroll
-  for (int i = 0; i < 3; i++) { x.V(i) = fma(w1, av[i], x.V(i)); x.U(i) = fma(w1, au[i], x.U(i)); }
-}
-
-// the same step with the state and the stage scratch in shared memory (FkState<NT, true>): identical
-// arithmetic in identical order, so both variants give bit-identical results
-template <int NT, typename RT>
-__device__ __forceinline__ void rk4_step(FkState<NT, true> &x, const double (&tau)[NT],
-                                         const double (&Kse)[3], const double (&Kbt)[3], double h,
-                                         const RT &rt0, const RT &rt1, const RT &rt2) {
-  const double hh = 0.5 * h, w1 = h * (1.0 / 6.0), w2 = h * (1.0 / 3.0);
-  double sv[3], su[3];
-#pragma unroll
-  for (int i = 0; i < 3; i++) { sv[i] = x.V(i); su[i] = x.U(i); x.AV(i) = 0.0; x.AU(i) = 0.0; }
-#pragma unroll
-  for (int i = 0; i < 9; i++) { x.SR(i) = x.R(i); x.AR(i) = 0.0; }
-
-#pragma unroll 1
-  for (int stage = 0; stage < 4; stage++) {
-    const bool outer = (stage == 0) || (stage == 3);
-    const RT rt = (stage == 0) ? rt0 : ((stage == 3) ? rt2 : rt1);
-    const double wq = outer ? w1 : w2;     // quadrature weight
-    const double wk = outer ? 1.0 : 2.0;   // slope weight
-    const double a = (stage == 2) ? h : hh;
-    double vd[3], ud[3], sig[NT];
-    // compiler barriers: without them the stored stage values are forwarded in registers across the derivative
-    // evaluation (store-to-load forwarding), which is exactly the register pressure this variant is meant to shed
-    asm volatile("" ::: "memory");
-    vu_dot<NT, RT>(rt, tau, Kse, Kbt, sv, su, vd, ud, sig);
-    asm volatile("" ::: "memory");
-    double sR[9], Rd[9];
-#pragma unroll
-    for (int i = 0; i < 9; i++) sR[i] = x.SR(i);
-#pragma unroll
-    for (int i = 0; i < 3; i++)
-      x.P(i) = fma(wq, fma(sR[i], sv[0], fma(sR[i + 3], sv[1], sR[i + 6] * sv[2])), x.P(i));
-    {
-      const double vv = fma(sv[0], sv[0], fma(sv[1], sv[1], sv[2] * sv[2]));
-#if FK_FAST_PRIMS
-      x.LB() = fma(wq, vv * rsqrt_fast(vv), x.LB());
-#else
-      x.LB() = fma(wq, sqrt(vv), x.LB());
-#endif
-    }
-#pragma unroll
-    for (int j = 0; j < NT; j++) x.LI(j) = fma(wq, sig[j], x.LI(j));
-#pragma unroll
-    for (int i = 0; i < 3; i++) {
-      Rd[i] = fma(sR[i + 3], su[2], -sR[i + 6] * su[1]);
-      Rd[i + 3] = fma(sR[i + 6], su[0], -sR[i] * su[2]);
-      Rd[i + 6] = fma(sR[i], su[1], -sR[i + 3] * su[0]);
-    }
-#pragma unroll
-    for (int i = 0; i < 9; i++) { x.AR(i) = fma(wk, Rd[i], x.AR(i)); x.SR(i) = fma(a, Rd[i], x.R(i)); }
-#pragma unroll
-    for (int i = 0; i < 3; i++) {
-      x.AV(i) = fma(wk, vd[i], x.AV(i)); x.AU(i) = fma(wk, ud[i], x.AU(i));
-      sv[i] = fma(a, vd[i], x.V(i)); su[i] = fma(a, ud[i], x.U(i));
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 9; i++) x.R(i) = fma(w1, x.AR(i), x.R(i));
-#pragma unroll
-  for (int i = 0; i < 3; i++) { x.V(i) = fma(w1, x.AV(i), x.V(i)); x.U(i) = fma(w1, x.AU(i), x.U(i)); }
+  for (int i = 0; i < 3; i++) { x.v[i] = fma(w1, av[i], x.v[i]); x.u[i] = fma(w1, au[i], x.u[i]); }
 }
 
 struct RotZ {
@@ -511,11 +352,11 @@ struct RotZ {
   int on;
 };
 
-template <int NT, bool SM>
+template <int NT>
 __device__ __forceinline__ void emit_node(const irt_fk_outputs &o, int64_t row_base, int k,
-                                          double t, const FkState<NT, SM> &x, const RotZ &rz) {
+                                          double t, const FkState<NT> &x, const RotZ &rz) {
   const int64_t row = row_base + k;
-  const double p0 = x.P(0), p1 = x.P(1), p2 = x.P(2);
+  const double p0 = x.p[0], p1 = x.p[1], p2 = x.p[2];
   double px = p0, py = p1;
   if (rz.on) {
     px = rz.c * p0 - rz.s * p1;
@@ -530,7 +371,7 @@ __device__ __forceinline__ void emit_node(const irt_fk_outputs &o, int64_t row_b
     double *dst = o.R + row * 9;
 #pragma unroll
     for (int j = 0; j < 3; j++) {
-      double r0 = x.R(3 * j), r1 = x.R(3 * j + 1);
+      double r0 = x.R[3 * j], r1 = x.R[3 * j + 1];
       if (rz.on) {
         dst[3 * j] = rz.c * r0 - rz.s * r1;
         dst[3 * j + 1] = rz.s * r0 + rz.c * r1;
@@ -538,7 +379,7 @@ __device__ __forceinline__ void emit_node(const irt_fk_outputs &o, int64_t row_b
         dst[3 * j] = r0;
         dst[3 * j + 1] = r1;
       }
-      dst[3 * j + 2] = x.R(3 * j + 2);
+      dst[3 * j + 2] = x.R[3 * j + 2];
     }
   }
 }
@@ -594,21 +435,18 @@ struct FkArgs {
   int use_const;          // c_fk_tab holds this robot's routing table
 };
 
-#define FK_KERNEL_BOUNDS __launch_bounds__(SM ? FK_SM_THREADS : FK_THREADS, SM ? FK_SM_MIN_BLOCKS : FK_MIN_BLOCKS)
-
-// Persistent kernel: FK_MIN_BLOCKS CTAs per SM stage the routing table once, then every WARP fetches the next
+// Persistent kernel: FK_BLOCKS_PER_SM CTAs per SM stage the routing table once, then every WARP fetches the next
 // 32 configurations of the bucket order from a global counter until the batch is done (no CTA-wide barrier after
 // the staging, no tail of half-empty CTAs, and the batch size may live in device memory: K2's bisection rounds
 // launch this kernel without the host knowing how many samples a round has).
-template <int NT, bool RETRACT, bool SM>
-__global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkArgs a) {
-  constexpr int THREADS = SM ? FK_SM_THREADS : FK_THREADS;
+template <int NT, bool RETRACT>
+__global__ void __launch_bounds__(FK_THREADS, FK_BLOCKS_PER_SM) fk_rk4_fp64_kernel(const RobotDev rb, const FkArgs a) {
   extern __shared__ double smem[];
   double *tab = smem;                                // [n_table][NT][6]
   double *head = smem + (size_t)rb.n_table * NT * 6; // [4][NT][6]
   int64_t lo = 0, n = a.n;
   if (a.range) { lo = a.range[0]; n = (int64_t)a.range[1] - lo; }
-  if (n <= 0 || (int64_t)blockIdx.x * THREADS >= n) return;   // the other CTAs cover the batch
+  if (n <= 0 || (int64_t)blockIdx.x * FK_THREADS >= n) return;   // the other CTAs cover the batch
   for (int i = threadIdx.x; i < rb.n_table * NT * 6; i += blockDim.x) tab[i] = rb.table[i];
   for (int i = threadIdx.x; i < 4 * NT * 6; i += blockDim.x) head[i] = rb.head[i];
   __syncthreads();
@@ -618,7 +456,6 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
   const double Kbt[3] = {rb.Kbt[0], rb.Kbt[1], rb.Kbt[2]};
   const int lane = threadIdx.x & 31;
 
-#if FK_PERSIST
   // every WARP fetches the next 32 configurations of the bucket order from a global counter
 #pragma unroll 1
   for (;;) {
@@ -627,15 +464,6 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
   wbase = __shfl_sync(0xffffffffu, wbase, 0);
   if (wbase >= n) break;
   const int64_t gi = wbase + lane;
-#else
-  // block-strided: with a host-known batch the grid has one CTA per 128 configurations (the hardware hands
-  // CTAs to SMs as slots free up, and the warps of a CTA walk the code in step: instruction-cache friendly);
-  // with a device-side batch size (K2) a resident grid strides over it
-#pragma unroll 1
-  for (int64_t blk = blockIdx.x; blk * THREADS < n; blk += gridDim.x) {
-  const int64_t gi = blk * THREADS + threadIdx.x;
-  (void)lane;
-#endif
   const bool in_range = gi < n;
   const int64_t rel = in_range ? (a.perm ? (int64_t)a.perm[gi] : gi) : 0;
   const int64_t cfg = lo + rel;
@@ -684,17 +512,16 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
   }
   const bool degenerate = active && (s_start == rb.L);  // TendonRobot.cpp:361-372
 
-  FkState<NT, SM> x;
-  if constexpr (SM) x.sm = head + 4 * NT * 6 + threadIdx.x;   // [fk_sm_slots][FK_SM_THREADS] behind the tables
+  FkState<NT> x;
 #pragma unroll
-  for (int i = 0; i < 3; i++) { x.P(i) = 0; x.V(i) = 0; x.U(i) = 0; }
+  for (int i = 0; i < 3; i++) { x.p[i] = 0; x.v[i] = 0; x.u[i] = 0; }
 #pragma unroll
-  for (int i = 0; i < 9; i++) x.R(i) = 0;
-  x.R(0) = x.R(4) = x.R(8) = 1.0;
-  x.V(2) = 1.0;
-  x.LB() = 0;
+  for (int i = 0; i < 9; i++) x.R[i] = 0;
+  x.R[0] = x.R[4] = x.R[8] = 1.0;
+  x.v[2] = 1.0;
+  x.L = 0;
 #pragma unroll
-  for (int j = 0; j < NT; j++) x.LI(j) = 0;
+  for (int j = 0; j < NT; j++) x.Li[j] = 0;
 
   int iters = 0, nsteps = 0;
   double u0[3] = {0, 0, 0}, v0[3] = {0, 0, 1};
@@ -783,7 +610,7 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
       u[0] = un0; u[1] = un1; u[2] = un2;
     }
 #pragma unroll
-    for (int i = 0; i < 3; i++) { x.V(i) = v0[i] = v[i]; x.U(i) = u0[i] = u[i]; }
+    for (int i = 0; i < 3; i++) { x.v[i] = v0[i] = v[i]; x.u[i] = u0[i] = u[i]; }
 
     // ---- convergence flag: calc_point_forces at the base, R = I (TendonRobot.cpp:188-217) --
     {
@@ -810,7 +637,7 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
   // Head steps, then the regular steps node q -> node q-1.  All steps run through ONE rk4_step call site in
   // a loop that is end-aligned across the warp, so that every lane is at the same regular step q in the
   // same iteration (table reads are broadcasts).
-  if (run) emit_node<NT, SM>(o, row_base, 0, s_start, x, rz);
+  if (run) emit_node<NT>(o, row_base, 0, s_start, x, rz);
   {
     const int T = integ ? (K - 1 + nhead) : 0;
     // the warp's step count: every lane runs the loop the same number of times (lanes that do not integrate idle
@@ -820,16 +647,14 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
 #pragma unroll 1
     for (int j = 0; j < Tmax; j++) {
       const int q = Tmax - j;  // regular step q: node q -> node q-1 (1 <= q <= K-1)
-#if FK_CONST_TABLE
       // every lane of the warp takes the regular step q (the common case: buckets are warps of equal step
       // counts): the routing rows come from constant memory by a warp-uniform index, the step size is uniform
-      if (!SM && a.use_const && __all_sync(0xffffffffu, integ && q <= K - 1)) {
+      if (a.use_const && __all_sync(0xffffffffu, integ && q <= K - 1)) {
         const int b0 = 2 * q * NT * 6;
         rk4_step<NT, RtConst>(x, tau, Kse, Kbt, rb.dL, RtConst{b0}, RtConst{b0 - NT * 6}, RtConst{b0 - 2 * NT * 6});
-        emit_node<NT, SM>(o, row_base, K - q + 1, rb.node_t[q - 1], x, rz);
+        emit_node<NT>(o, row_base, K - q + 1, rb.node_t[q - 1], x, rz);
         continue;
       }
-#endif
       if (integ && q <= K - 1 + nhead) {
         const double *p0, *p1, *p2;
         double h;
@@ -852,7 +677,7 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
           emit_idx = -1;
         }
         rk4_step<NT, RtPtr>(x, tau, Kse, Kbt, h, RtPtr{p0}, RtPtr{p1}, RtPtr{p2});
-        if (emit_idx >= 0) emit_node<NT, SM>(o, row_base, emit_idx, rb.node_t[K - emit_idx], x, rz);
+        if (emit_idx >= 0) emit_node<NT>(o, row_base, emit_idx, rb.node_t[K - emit_idx], x, rz);
       }
     }
   }
@@ -861,7 +686,7 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
   int npts = 0;
   if (degenerate) {
     npts = 1;
-    emit_node<NT, SM>(o, row_base, 0, s_start, x, rz);  // p = 0, R = I, v = e3, u = 0
+    emit_node<NT>(o, row_base, 0, s_start, x, rz);  // p = 0, R = I, v = e3, u = 0
   } else if (run) {
     npts = K + 1;
   }
@@ -871,18 +696,18 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
     const double Lhome = degenerate ? 0.0 : (rb.L - sh);
 #pragma unroll
     for (int j = 0; j < NT; j++) {
-      const double dl = Lhome * rb.home_factor[j] - x.LI(j);
+      const double dl = Lhome * rb.home_factor[j] - x.Li[j];
       if (dl < rb.min_length[j] || rb.max_length[j] < dl) flags |= IRT_FLAG_LENGTH_LIMIT;
     }
   }
   if (o.npts) o.npts[cfg] = npts;
-  if (o.L) o.L[cfg] = x.LB();
+  if (o.L) o.L[cfg] = x.L;
   if (o.L_i) {
 #pragma unroll
-    for (int j = 0; j < NT; j++) o.L_i[cfg * NT + j] = x.LI(j);
+    for (int j = 0; j < NT; j++) o.L_i[cfg * NT + j] = x.Li[j];
   }
   if (o.tip) {
-    const double p0 = x.P(0), p1 = x.P(1), p2 = x.P(2);
+    const double p0 = x.p[0], p1 = x.p[1], p2 = x.p[2];
     double px = p0, py = p1;
     if (rz.on) { px = rz.c * p0 - rz.s * p1; py = rz.s * p0 + rz.c * p1; }
     o.tip[cfg * 3] = px; o.tip[cfg * 3 + 1] = py; o.tip[cfg * 3 + 2] = p2;
@@ -890,7 +715,7 @@ __global__ void FK_KERNEL_BOUNDS fk_rk4_fp64_kernel(const RobotDev rb, const FkA
   if (o.uv) {
     double *d = o.uv + cfg * 12;
 #pragma unroll
-    for (int i = 0; i < 3; i++) { d[i] = u0[i]; d[3 + i] = x.U(i); d[6 + i] = v0[i]; d[9 + i] = x.V(i); }
+    for (int i = 0; i < 3; i++) { d[i] = u0[i]; d[3 + i] = x.u[i]; d[6 + i] = v0[i]; d[9 + i] = x.v[i]; }
   }
   if (o.flags) o.flags[cfg] = flags;
   if (o.iters) o.iters[cfg] = iters;
@@ -992,19 +817,14 @@ __global__ void fk_bucket_scatter_kernel(const int32_t *__restrict__ keys, int64
   }
 }
 
-template <int NT, bool RETRACT, bool SM>
+template <int NT, bool RETRACT>
 int launch_k(irt_ctx *ctx, const RobotDev &d, const FkArgs &a, size_t smem, cudaStream_t st) {
-  constexpr int THREADS = SM ? FK_SM_THREADS : FK_THREADS;
-  int64_t blocks = (a.n + THREADS - 1) / THREADS;
-  const int64_t resident = (int64_t)ctx->sm_count * (SM ? FK_SM_MIN_BLOCKS : FK_MIN_BLOCKS);
-#if FK_PERSIST
+  int64_t blocks = (a.n + FK_THREADS - 1) / FK_THREADS;
+  const int64_t resident = (int64_t)ctx->sm_count * FK_BLOCKS_PER_SM;
   if (blocks > resident) blocks = resident;
-#else
-  if (a.range && blocks > resident) blocks = resident;   // batch size only known on the device: strided grid
-#endif
-  auto k = fk_rk4_fp64_kernel<NT, RETRACT, SM>;
+  auto k = fk_rk4_fp64_kernel<NT, RETRACT>;
   IRT_CUDA(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k<<<(unsigned)blocks, THREADS, smem, st>>>(d, a);
+  k<<<(unsigned)blocks, FK_THREADS, smem, st>>>(d, a);
   IRT_LAUNCHED(ctx);
   IRT_CUDA(ctx, cudaGetLastError());
   return IRT_OK;
@@ -1014,15 +834,7 @@ template <int NT>
 int launch_nt(irt_ctx *ctx, const irt_robot *rb, const FkArgs &a, cudaStream_t st) {
   const RobotDev &d = rb->dev;
   const size_t smem = ((size_t)d.n_table + 4) * NT * 6 * sizeof(double);
-#if FK_SMEM_VARIANT
-  // state in shared memory, 12 warps per SM: when the slots fit beside the routing table
-  const size_t smem_sm = smem + (size_t)fk_sm_slots<NT>() * FK_SM_THREADS * sizeof(double);
-  if (ctx->fk_smem && smem_sm * FK_SM_MIN_BLOCKS <= 226 * 1024)
-    return d.enable_retraction ? launch_k<NT, true, true>(ctx, d, a, smem_sm, st)
-                               : launch_k<NT, false, true>(ctx, d, a, smem_sm, st);
-#endif
-  return d.enable_retraction ? launch_k<NT, true, false>(ctx, d, a, smem, st)
-                             : launch_k<NT, false, false>(ctx, d, a, smem, st);
+  return d.enable_retraction ? launch_k<NT, true>(ctx, d, a, smem, st) : launch_k<NT, false>(ctx, d, a, smem, st);
 }
 
 }  // namespace
@@ -1098,7 +910,6 @@ int fk_launch(irt_ctx *ctx, const irt_robot *rb, const double *d_states, int64_t
     a.keys = keys;
   }
   a.use_const = 0;
-#if FK_CONST_TABLE
   // The kernel's fast path reads the routing table from constant memory, which is ONE array per device and process:
   // it is tagged with the robot it holds.  A launch for another robot waits for everything that may still read the
   // old table (device-wide, rare: applications use one robot), uploads, and the lock is held across the launch so
@@ -1107,7 +918,7 @@ int fk_launch(irt_ctx *ctx, const irt_robot *rb, const double *d_states, int64_t
   static unsigned long long ct_owner[64] = {};
   std::unique_lock<std::mutex> ct_lock(ct_mutex, std::defer_lock);
   const size_t tab_doubles = (size_t)d.n_table * d.n_tendons * 6;
-  if (tab_doubles <= (size_t)FK_CT_DOUBLES && ctx->device >= 0 && ctx->device < 64 && !ctx->fk_smem) {
+  if (tab_doubles <= (size_t)FK_CT_DOUBLES && ctx->device >= 0 && ctx->device < 64) {
     ct_lock.lock();
     if (ct_owner[ctx->device] != rb->uid) {
       IRT_CUDA(ctx, cudaDeviceSynchronize());
@@ -1118,7 +929,6 @@ int fk_launch(irt_ctx *ctx, const irt_robot *rb, const double *d_states, int64_t
     }
     a.use_const = 1;
   }
-#endif
   switch (d.n_tendons) {
     case 1: return launch_nt<1>(ctx, rb, a, st);
     case 2: return launch_nt<2>(ctx, rb, a, st);

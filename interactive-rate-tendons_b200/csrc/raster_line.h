@@ -15,9 +15,6 @@
 #define RL_HD inline
 #define RL_HDI inline
 #endif
-#ifndef RS_FAST_TRAVERSAL
-#define RS_FAST_TRAVERSAL 1
-#endif
 // hooks of the host harness (count which path a segment took); nothing on the device
 #ifndef RL_ON_FAST_PATH_DONE
 #define RL_ON_FAST_PATH_DONE
@@ -80,7 +77,6 @@ RL_HD void add_line(const Grid &g, Sink &sink, const D3 &a, const D3 &b) {
   if (entered) sink.cell(Axi, Ayi, Azi);
   D3 U = {B.x - A.x, B.y - A.y, B.z - A.z};
   const double z = (U.x * U.x + U.y * U.y) + U.z * U.z;  // Eigen normalized()
-#if RS_FAST_TRAVERSAL
   // Division-free traversal.  The reference's ray parameters are t_axis(k) = (e_axis + k) * n / |U_axis| (U the
   // un-normalised direction, n its norm, k the steps already taken on that axis), so every comparison between
   // two of them is a comparison of cross products (e_x + k_x) |U_y| <> (e_y + k_y) |U_x|: no square root, no
@@ -128,7 +124,6 @@ RL_HD void add_line(const Grid &g, Sink &sink, const D3 &a, const D3 &b) {
       }
     }
   }
-#endif
   RL_ON_LITERAL_PATH
   bool entered_l = entered;
   if (z > 0.0) {

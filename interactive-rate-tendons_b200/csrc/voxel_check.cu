@@ -17,7 +17,6 @@
 // (behind the occupancy bitmap) is non-zero sets one bit in a shared-memory hit bitmap, and each
 // thread then tests the bits of the one set it owns; the word is one __ballot_sync per warp: no
 // global atomics, no memset, no search, no per-set divergence (details at the kernel).
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -74,6 +73,10 @@ __global__ void count_nonzero_kernel(const uint64_t *__restrict__ blocks, int64_
 constexpr int K3_CHUNK_LEAVES = 32768;                      // hit-bitmap capacity per buffer (4 KiB)
 constexpr int K3_BM_WORDS = K3_CHUNK_LEAVES / 32 + 2;       // +1 straddle word, +1 pad
 constexpr int K3_GATHER_TILES = 256;                         // staged verdict words per CTA: 8 KiB
+// staged tiles per P2P flush: peer stores trickle out while the sweep runs, so the fence at the end of a CTA only
+// waits for its last few
+constexpr int K3_GATHER_FLUSH_TILES = 4;
+static_assert(K3_GATHER_FLUSH_TILES <= K3_GATHER_TILES, "a flush cannot hold more tiles than are staged");
 constexpr int K3_SMEM_FIXED_WORDS = 3 * K3_BM_WORDS + (3 * K3_BM_WORDS & 1) + 2 * 2 * (K3_THREADS + 2);
 
 // predicated 8-byte read-only load: the four environment look-ups of a quad are issued back to back
@@ -109,16 +112,10 @@ __device__ __forceinline__ ulonglong2 ld_stream(const ulonglong2 *p) {
 // epoch flag on every peer and waits for the peers' flags.  No NCCL call, no extra kernel between the sweep and
 // its consumers.
 constexpr int IRT_MAX_PEERS = 16;
-// 1: a CTA publishes its peer stores towards the LAST CTA with a gpu-scope fence and only the last CTA pays a
-// system-scope fence before the flags (-6 us per sweep: MEMBAR.SYS twice in a row on the critical path was ~10 us);
-// 0: every CTA fences at system scope
-#ifndef K3_CTA_FENCE_GPU
-#define K3_CTA_FENCE_GPU 1
-#endif
 struct XchgDev {
   uint32_t *peer[IRT_MAX_PEERS];  // base of every rank's buffer as mapped in THIS process (own: local)
   int world, rank, parity;
-  int flush_tiles;                // staged tiles per P2P flush (<= K3_GATHER_TILES)
+  int flush_tiles;                // staged tiles per P2P flush (the host sets K3_GATHER_FLUSH_TILES)
   int64_t slot_words;             // words every rank contributes
   uint32_t epoch;
   unsigned int *done;             // local: [0] CTAs done, [1] error word, [2] dynamic tile counter
@@ -148,11 +145,10 @@ __device__ __forceinline__ void xchg_signal(const XchgDev &x) {
   __shared__ int s_last;
   __syncthreads();
   if (threadIdx.x == 0) {
-#if K3_CTA_FENCE_GPU
+    // a CTA publishes its peer stores towards the LAST CTA with a gpu-scope fence and only the last CTA pays a
+    // system-scope fence before the flags (-6 us per sweep: MEMBAR.SYS twice in a row on the critical path was
+    // ~10 us)
     __threadfence();
-#else
-    __threadfence_system();
-#endif
     const unsigned prev = atomicAdd(x.done, 1u);
     s_last = (prev == gridDim.x - 1);
     if (s_last) {
@@ -722,7 +718,6 @@ struct irt_xchg {
   unsigned int *d_done = nullptr;     // [0] CTA counter, [1] error word, [2] dynamic tile counter
   uint32_t epoch = 0;
   bool connected = false;
-  int flush_tiles = 4;                // staged tiles per P2P flush (IRT_K3_GATHER_FLUSH, read once at creation)
 };
 
 int irt_xchg_create(irt_ctx *ctx, int rank, int world, int64_t slot_words, irt_xchg **out) {
@@ -741,13 +736,6 @@ int irt_xchg_create(irt_ctx *ctx, int rank, int world, int64_t slot_words, irt_x
   cudaMemset(x->d_done, 0, 64);
   x->peer[rank] = x->local;
   x->connected = (world == 1);
-  {
-    // peer stores trickle out while the sweep runs (every flush_tiles tiles), so the fence at the end of
-    // a CTA only waits for its last few; tuning knob IRT_K3_GATHER_FLUSH
-    const char *fl = getenv("IRT_K3_GATHER_FLUSH");
-    const int f = (fl && atoi(fl) > 0) ? atoi(fl) : 4;
-    x->flush_tiles = f > K3_GATHER_TILES ? K3_GATHER_TILES : f;
-  }
   *out = x;
   return IRT_OK;
 }
@@ -810,7 +798,7 @@ int irt_check_sets_allgather_dev(irt_ctx *ctx, const irt_setstore *store, const 
   for (int r = 0; r < x->world; r++) xd.peer[r] = x->peer[r];
   xd.world = x->world; xd.rank = x->rank; xd.parity = (int)(x->epoch & 1u);
   xd.slot_words = x->slot_words; xd.epoch = x->epoch; xd.done = x->d_done;
-  xd.flush_tiles = x->flush_tiles;
+  xd.flush_tiles = K3_GATHER_FLUSH_TILES;
   int rc = check_sets_impl(ctx, store, env, begin, end, nullptr, nullptr, st, &xd);
   if (rc) return rc;
   // (the kernel's last CTA has waited for every peer's flag: the gathered array is complete when it ends)

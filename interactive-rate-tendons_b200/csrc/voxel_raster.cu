@@ -85,12 +85,8 @@ struct Timeline {
 };
 
 constexpr int RS_WARPS = 4;
-#ifndef ES_MINB
-#define ES_MINB 4   // resident CTAs per SM of the subdivision test
-#endif
-#ifndef RS_MINB
-#define RS_MINB 6   // resident CTAs per SM the main raster pass is compiled for (80 registers; 5 -> 6: -10 %, 7 and 8: no further gain)
-#endif
+constexpr int ES_MINB = 4;   // resident CTAs per SM of the subdivision test
+constexpr int RS_MINB = 6;   // resident CTAs per SM the main raster pass is compiled for (80 registers; 5 -> 6: -10 %, 7 and 8: no further gain)
 constexpr int RS_HLOG_SMALL = 8;     // main pass: 256 hash entries per warp (a set rarely exceeds ~150 blocks)
 constexpr int RS_HLOG_BIG = 12;      // fallback pass for the sets that overflow it: 4096 entries, 1 warp per CTA
 constexpr int RS_SLOT = 1 << RS_HLOG_SMALL;   // slot capacity of the main pass
@@ -197,9 +193,7 @@ struct HashSink {
 // lanes with equal keys merge their masks with a shuffle reduction and ONE lane per distinct key touches the
 // hash -- instead of 4-8 lanes contending for the same shared-memory word with atomicCAS / atomicOr.
 constexpr int RS_PAIRS = 3;
-#ifndef RS_SEGS
-#define RS_SEGS 2   // consecutive segments a lane handles per warp iteration
-#endif
+constexpr int RS_SEGS = 2;   // consecutive segments a lane handles per warp iteration
 struct PairSink {
   const WarpHash &h;
   BlockAcc acc;

@@ -1,4 +1,4 @@
-"""Static model of K1's RK4 stage loop from its SASS (cuobjdump -sass of fk.o, the fk_rk4_fp64_kernel<6,1,0> function):
+"""Static model of K1's RK4 stage loop from its SASS (cuobjdump -sass of fk.o, the fk_rk4_fp64_kernel<6,1> function):
 
   * the scheduled stall counts (control codes) of the loop body: the time ONE warp needs per stage if nothing else
     ran -- against the 2 cycles per FP64 warp instruction the pipe needs;
@@ -8,8 +8,8 @@
     max(rt_pipe, #even_distinct, #odd_distinct)).  The ratio of the two sums is the ceiling of
     sm__pipe_fp64_cycles_active for this instruction stream.
 
-usage:  cuobjdump -sass interactive-rate-tendons_b200/csrc/fk.o | awk '/Function :.*fk_rk4_fp64_kernelILi6ELb1ELb0/{f=1}
-        f&&/Function :/&&!/fk_rk4_fp64_kernelILi6ELb1ELb0/{f=0} f' > /tmp/fk.sass;  python tools/sass_fp64_rf_model.py /tmp/fk.sass
+usage:  cuobjdump -sass interactive-rate-tendons_b200/csrc/fk.o | awk '/Function :.*fk_rk4_fp64_kernelILi6ELb1E/{f=1}
+        f&&/Function :/&&!/fk_rk4_fp64_kernelILi6ELb1E/{f=0} f' > /tmp/fk.sass;  python tools/sass_fp64_rf_model.py /tmp/fk.sass
 """
 import re
 import sys
