@@ -178,8 +178,8 @@ def grid(nm, s, L, dL):
 
 
 def fk(rb, state, mp=None, v0u0=None):
-    """Returns dict(t, p, R (row-major 3x3 lists), L, L_i).  `v0u0` lets the caller impose the
-    initial condition (to compare integrators independently of the fixed-point stop rule)."""
+    """Returns dict(t, p, R (row-major 3x3 lists), L, L_i, v0, u0, v_f, u_f, iters).  `v0u0` lets the
+    caller impose the initial condition (to compare integrators independently of the fixed-point stop rule)."""
     nm = Num(mp)
     f = nm.f
     N = len(rb["C"])
@@ -240,4 +240,4 @@ def fk(rb, state, mp=None, v0u0=None):
         out_p = [[dot(Rz[i], q) for i in range(3)] for q in out_p]
         out_R = [[[sum(Rz[i][k] * Rm[k][j] for k in range(3)) for j in range(3)] for i in range(3)]
                  for Rm in out_R]
-    return dict(t=ts, p=out_p, R=out_R, L=y[4], L_i=y[5], v0=v, u0=u, iters=iters)
+    return dict(t=ts, p=out_p, R=out_R, L=y[4], L_i=y[5], v0=v, u0=u, v_f=y[2], u_f=y[3], iters=iters)
