@@ -260,6 +260,17 @@ int irt_setstore_import(irt_ctx *ctx, irt_setstore *s, int64_t n_sets, const uin
                         const uint32_t *keys, const uint64_t *bits);
 int irt_setstore_export(irt_ctx *ctx, const irt_setstore *s, uint64_t *offsets, uint32_t *keys,
                         uint64_t *bits);
+/* Append sets [begin, end) of src to the end of dst, in index order.  keep_words (host, may be NULL = keep all):
+ * set begin+i is appended iff bit i % 32 of word i / 32 is set.  dst's existing sets, offsets, keys and bits are
+ * unchanged; afterwards dst equals irt_setstore_import of the concatenated CSR, bit for bit.  Synchronous.
+ * IRT_ERR_INVALID_ARGUMENT: dst == src, NULL handles, grids that differ (Ng, lim, inv_rot), begin/end outside
+ * [0, num_sets(src)] or begin > end, stores of another context's device.  An empty range or an all-clear mask is a
+ * no-op.  On any error dst is unchanged.  Device views of dst (irt_setstore_device_ptrs) are invalidated.
+ * The batch form of the reference's compute-if-absent voxelizeVertex / voxelizeEdge (VoxelCachedLazyPRM.cpp:
+ * 2803-2837, 2879-2902) and of the per-increment caches of createRoadmap(N) (.cpp:1380-1561): voxelise the new
+ * items into a scratch store, then append the kept ones (INTEGRATION.md section B). */
+int irt_setstore_append(irt_ctx *ctx, irt_setstore *dst, const irt_setstore *src, int64_t begin, int64_t end,
+                        const uint32_t *keep_words);
 /* device views (valid until the store is next modified) */
 int irt_setstore_device_ptrs(const irt_setstore *s, const uint64_t **d_offsets,
                              const uint32_t **d_keys, const uint64_t **d_bits);

@@ -111,7 +111,7 @@ ABI_SYMBOLS = [
     "irt_env_add_primitives",
     "irt_env_dilate", "irt_env_dilate_sphere", "irt_env_remove_interior", "irt_env_download",
     "irt_setstore_create", "irt_setstore_destroy", "irt_setstore_num_sets",
-    "irt_setstore_num_blocks", "irt_setstore_import", "irt_setstore_export",
+    "irt_setstore_num_blocks", "irt_setstore_import", "irt_setstore_export", "irt_setstore_append",
     "irt_setstore_device_ptrs", "irt_morton_key", "irt_morton_decode",
     "irt_voxelize_vertices", "irt_voxelize_shapes", "irt_voxelize_edges", "irt_voxelize_edges_until_invalid", "irt_voxelize_edges_indexed",
     "irt_valid_segment_count",
@@ -177,6 +177,7 @@ def lib():
         "irt_setstore_num_blocks": (i64, [vp]),
         "irt_setstore_import": (i32, [vp, vp, i64, vp, vp, vp]),
         "irt_setstore_export": (i32, [vp, vp, vp, vp, vp]),
+        "irt_setstore_append": (i32, [vp, vp, vp, i64, i64, vp]),
         "irt_setstore_device_ptrs": (i32, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
         "irt_morton_key": (u32, [i32, i32, i32, i32]),
         "irt_morton_decode": (None, [u32, i32, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]),
@@ -565,6 +566,19 @@ class SetStore:
         bits = np.zeros(max(nb, 1), dtype=np.uint64)
         self.ctx.check(self.ctx.L.irt_setstore_export(self.ctx.h, self.h, _ptr(offsets), _ptr(keys), _ptr(bits)))
         return offsets, keys[:nb], bits[:nb]
+
+    def append(self, src, keep=None, begin=0, end=None):
+        """Append sets [begin, end) of the store `src` after this store's last set, in index order; keep (bool[end -
+        begin], optional) selects the sets that are appended.  The sets already here stay as they are."""
+        end = src.num_sets if end is None else end
+        words = None
+        if keep is not None:
+            keep = np.asarray(keep, dtype=bool)
+            if keep.shape != (max(end - begin, 0),):
+                raise IrtError(IRT_ERR_INVALID_ARGUMENT, "keep must hold one flag per set of the range")
+            words = pack_mask(keep)
+        self.ctx.check(self.ctx.L.irt_setstore_append(self.ctx.h, self.h, src.h, begin, end,
+                                                      _ptr(words) if words is not None else None))
 
     def voxelize_vertices(self, robot, states):
         """precomputeVertexVoxelCache: FK + is_valid_shape + voxelize for every state.

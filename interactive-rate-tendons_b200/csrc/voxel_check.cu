@@ -20,6 +20,8 @@
 #include <cstring>
 #include <vector>
 
+#include <cub/device/device_scan.cuh>
+
 #include "common.cuh"
 
 namespace {
@@ -406,6 +408,52 @@ int ensure_store_capacity(irt_ctx *ctx, irt_setstore *s, int64_t n_sets, int64_t
   return IRT_OK;
 }
 
+// ---- append: stream compaction of a CSR range onto the end of another store ----------------------
+// (kept leaves before set i, kept sets before set i): the exclusive scan of these gives every kept set its leaf
+// position and its slot in the destination at once
+struct __align__(16) AppendPos {
+  unsigned long long leaves, sets;
+};
+struct AppendPosSum {
+  __device__ __forceinline__ AppendPos operator()(const AppendPos &a, const AppendPos &b) const {
+    return {a.leaves + b.leaves, a.sets + b.sets};
+  }
+};
+
+// pos[i] = (leaf count, 1) of set begin + i if it is kept, else (0, 0); pos[n] = (0, 0), so that the exclusive scan
+// of n + 1 entries ends with the totals
+__global__ void append_count_kernel(const uint64_t *__restrict__ src_off, int64_t begin, int64_t n,
+                                    const uint32_t *__restrict__ keep, AppendPos *__restrict__ pos) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i > n) return;
+  const bool kept = i < n && (!keep || ((keep[i >> 5] >> (i & 31)) & 1u));
+  pos[i] = kept ? AppendPos{src_off[begin + i + 1] - src_off[begin + i], 1ull} : AppendPos{0ull, 0ull};
+}
+
+// one warp per source set: a kept set's keys and bits go to their scanned position (lanes over its leaves, so every
+// load and store of a warp is one contiguous run) and its end offset to its slot
+constexpr int APPEND_THREADS = 256;
+__global__ void __launch_bounds__(APPEND_THREADS)
+append_gather_kernel(const uint64_t *__restrict__ src_off, const uint32_t *__restrict__ src_keys,
+                     const uint64_t *__restrict__ src_bits, int64_t begin, int64_t n,
+                     const AppendPos *__restrict__ pos, uint64_t dst_blocks, int64_t dst_sets,
+                     uint64_t *__restrict__ dst_off, uint32_t *__restrict__ dst_keys,
+                     uint64_t *__restrict__ dst_bits) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = (int64_t)gridDim.x * (APPEND_THREADS / 32);
+  for (int64_t i = (int64_t)blockIdx.x * (APPEND_THREADS / 32) + (threadIdx.x >> 5); i < n; i += warps) {
+    const AppendPos p = pos[i], q = pos[i + 1];
+    if (q.sets == p.sets) continue;   // masked out
+    const uint64_t len = q.leaves - p.leaves;
+    const uint64_t from = src_off[begin + i], to = dst_blocks + p.leaves;
+    for (uint64_t j = lane; j < len; j += 32) {
+      dst_keys[to + j] = src_keys[from + j];
+      dst_bits[to + j] = src_bits[from + j];
+    }
+    if (lane == 0) dst_off[dst_sets + 1 + (int64_t)p.sets] = dst_blocks + q.leaves;
+  }
+}
+
 }  // namespace
 
 // used by voxel_raster.cu after it has filled the store on the device
@@ -433,6 +481,27 @@ int setstore_grow_blocks(irt_ctx *ctx, irt_setstore *s, int64_t need_blocks, int
   s->d_keys = nk;
   s->d_bits = nb;
   s->cap_blocks = cap;
+  return IRT_OK;
+}
+
+// the same for the offsets array: room for need_sets sets (need_sets + 1 offsets), the first keep_sets + 1 offsets
+// kept; a store that never held an offsets array gets offsets[0] = 0
+static int setstore_grow_sets(irt_ctx *ctx, irt_setstore *s, int64_t need_sets, int64_t keep_sets,
+                              cudaStream_t st) {
+  if ((size_t)need_sets + 1 <= s->cap_sets) return IRT_OK;
+  size_t cap = s->cap_sets + s->cap_sets / 2;
+  if (cap < (size_t)need_sets + 1) cap = (size_t)need_sets + 1;
+  uint64_t *no = nullptr;
+  IRT_CUDA(ctx, cudaMalloc(&no, cap * 8));
+  if (s->d_offsets) {
+    IRT_CUDA(ctx, cudaMemcpyAsync(no, s->d_offsets, (size_t)(keep_sets + 1) * 8, cudaMemcpyDeviceToDevice, st));
+    IRT_CUDA(ctx, cudaStreamSynchronize(st));
+    cudaFree(s->d_offsets);
+  } else {
+    IRT_CUDA(ctx, cudaMemsetAsync(no, 0, 8, st));
+  }
+  s->d_offsets = no;
+  s->cap_sets = cap;
   return IRT_OK;
 }
 
@@ -634,6 +703,85 @@ int irt_setstore_device_ptrs(const irt_setstore *s, const uint64_t **d_offsets,
   if (d_offsets) *d_offsets = s->d_offsets;
   if (d_keys) *d_keys = s->d_keys;
   if (d_bits) *d_bits = s->d_bits;
+  return IRT_OK;
+}
+
+static bool same_grid(const irt_grid &a, const irt_grid &b) {
+  if (a.Ng != b.Ng) return false;
+  for (int i = 0; i < 6; i++)
+    if (a.lim[i] != b.lim[i]) return false;
+  for (int i = 0; i < 9; i++)
+    if (a.inv_rot[i] != b.inv_rot[i]) return false;
+  return true;
+}
+
+// count + scan (one CUB scan of (leaves, sets) pairs), one read-back of the totals to size the growth, then the
+// gather; dst is only written once every argument has been checked and the scratch is in place
+int irt_setstore_append(irt_ctx *ctx, irt_setstore *dst, const irt_setstore *src, int64_t begin, int64_t end,
+                        const uint32_t *keep_words) {
+  if (!ctx || !dst || !src) return IRT_ERR_INVALID_ARGUMENT;
+  if (dst == src) return irt_fail(ctx, IRT_ERR_INVALID_ARGUMENT, "a store cannot be appended to itself");
+  if (dst->ctx->device != ctx->device || src->ctx->device != ctx->device)
+    return irt_fail(ctx, IRT_ERR_INVALID_ARGUMENT, "stores of another device");
+  if (!same_grid(dst->grid, src->grid)) return irt_fail(ctx, IRT_ERR_INVALID_ARGUMENT, "the stores' grids differ");
+  if (begin < 0 || begin > end || end > src->n_sets)
+    return irt_fail(ctx, IRT_ERR_INVALID_ARGUMENT, "set range [%lld,%lld) outside [0,%lld]", (long long)begin,
+                    (long long)end, (long long)src->n_sets);
+  const int64_t n = end - begin;
+  const int64_t nwords = (n + 31) / 32;
+  if (keep_words) {
+    int64_t kept = 0;
+    for (int64_t w = 0; w < nwords; w++) {
+      uint32_t m = keep_words[w];
+      if (w == nwords - 1 && (n & 31)) m &= (1u << (n & 31)) - 1u;
+      kept += __builtin_popcount(m);
+    }
+    if (kept == 0) return IRT_OK;
+  }
+  if (n == 0) return IRT_OK;
+  IRT_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+
+  AppendPos *d_pos = nullptr;
+  size_t cub_bytes = 0;
+  IRT_CUDA(ctx, cub::DeviceScan::ExclusiveScan(nullptr, cub_bytes, d_pos, d_pos, AppendPosSum(),
+                                               AppendPos{0ull, 0ull}, n + 1, st));
+  const size_t pos_bytes = ((size_t)(n + 1) * sizeof(AppendPos) + 255) & ~(size_t)255;
+  const size_t cub_off = pos_bytes, keep_off = cub_off + ((cub_bytes + 255) & ~(size_t)255);
+  char *scr = (char *)ctx_scratch(ctx, keep_off + (size_t)nwords * 4 + 64);
+  if (!scr) return irt_fail(ctx, IRT_ERR_CUDA, "scratch alloc failed");
+  d_pos = (AppendPos *)scr;
+  uint32_t *d_keep = nullptr;
+  if (keep_words) {
+    d_keep = (uint32_t *)(scr + keep_off);
+    IRT_CUDA(ctx, cudaMemcpyAsync(d_keep, keep_words, (size_t)nwords * 4, cudaMemcpyHostToDevice, st));
+  }
+  const int T = 256;
+  append_count_kernel<<<(unsigned)((n + T) / T), T, 0, st>>>(src->d_offsets, begin, n, d_keep, d_pos);
+  IRT_LAUNCHED(ctx);
+  IRT_CUDA(ctx, cudaGetLastError());
+  IRT_CUDA(ctx, cub::DeviceScan::ExclusiveScan(scr + cub_off, cub_bytes, d_pos, d_pos, AppendPosSum(),
+                                               AppendPos{0ull, 0ull}, n + 1, st));
+  IRT_LAUNCHED(ctx);
+  AppendPos total;
+  IRT_CUDA(ctx, cudaMemcpyAsync(&total, d_pos + n, sizeof(total), cudaMemcpyDeviceToHost, st));
+  IRT_CUDA(ctx, cudaStreamSynchronize(st));
+
+  const int64_t new_sets = dst->n_sets + (int64_t)total.sets, new_blocks = dst->n_blocks + (int64_t)total.leaves;
+  int rc = setstore_grow_sets(ctx, dst, new_sets, dst->n_sets, st);
+  if (rc) return rc;
+  rc = setstore_grow_blocks(ctx, dst, new_blocks, dst->n_blocks, st);
+  if (rc) return rc;
+  int64_t blocks = (n + APPEND_THREADS / 32 - 1) / (APPEND_THREADS / 32);
+  if (blocks > (int64_t)ctx->sm_count * 16) blocks = (int64_t)ctx->sm_count * 16;
+  append_gather_kernel<<<(unsigned)blocks, APPEND_THREADS, 0, st>>>(
+      src->d_offsets, src->d_keys, src->d_bits, begin, n, d_pos, (uint64_t)dst->n_blocks, dst->n_sets,
+      dst->d_offsets, dst->d_keys, dst->d_bits);
+  IRT_LAUNCHED(ctx);
+  IRT_CUDA(ctx, cudaGetLastError());
+  rc = setstore_finalize(ctx, dst, new_sets, new_blocks, st);
+  if (rc) return rc;
+  IRT_CUDA(ctx, cudaStreamSynchronize(st));
   return IRT_OK;
 }
 

@@ -44,8 +44,10 @@
 
 #include "../../include/irt_b200.h"
 #ifdef IRT_TEST_OVER_STANDIN
-// built over the test-only stand-in of the C ABI (no GPU): irt_nnset_* come from a sequential host implementation
+// built over the test-only stand-in of the C ABI (no GPU): irt_nnset_* come from a sequential host implementation,
+// irt_setstore_append from the stand-in's export / import
 #include "../../tests/cpp/knn_standin.hpp"
+#include "../../tests/cpp/setstore_append_standin.hpp"
 #endif
 
 namespace irt {
@@ -1209,6 +1211,50 @@ public:
                                         estore_, eflags_.data(), nullptr, nullptr));
   }
   void precomputeVoxelCache() { precomputeVertexVoxelCache(); precomputeEdgeVoxelCache(); }
+  /// The batch form of the reference's compute-if-absent voxelizeVertex / voxelizeEdge (.cpp:2803-2837, 2879-2902)
+  /// over the items the caches lack (vertices and edges that roadmapIk / addMilestone added since the caches were
+  /// built): only they are voxelised, into scratch stores, and appended to the cached stores with their flags and
+  /// tips.  A cache that does not exist yet is built whole.  Afterwards the next sweep is one K3 launch over every
+  /// item.  Validity words are not touched.
+  void extendVoxelCache() {
+    const size_t S = robot_.state_size(), nv = states_.size(), ne = edges_.size();
+    if (vflags_.empty() || vflags_.size() > nv || tips_.size() < 3 * vflags_.size()) {
+      precomputeVertexVoxelCache();
+    } else if (vflags_.size() < nv) {
+      const size_t v0 = vflags_.size(), m = nv - v0;
+      std::vector<double> flat(m * S), tips(3 * m);
+      for (size_t i = 0; i < m; i++) std::copy(states_[v0 + i].begin(), states_[v0 + i].end(), flat.begin() + i * S);
+      std::vector<uint32_t> fl(m);
+      std::shared_ptr<irt_setstore> scratch = scratch_store();
+      irt::check(ctx_, irt_voxelize_vertices(ctx_, robot_.handle(), flat.data(), (int)S, (int64_t)m, scratch.get(),
+                                             fl.data(), tips.data()));
+      irt::check(ctx_, irt_setstore_append(ctx_, vstore_, scratch.get(), 0, (int64_t)m, nullptr));
+      vflags_.insert(vflags_.end(), fl.begin(), fl.end());
+      if (tips_.size() == 3 * v0) {
+        tips_.insert(tips_.end(), tips.begin(), tips.end());   // appended rows: the k-NN copy appends them too
+      } else if (tips_.size() != 3 * nv || !std::equal(tips.begin(), tips.end(), tips_.begin() + 3 * v0)) {
+        tips_.resize(3 * v0);
+        tips_.insert(tips_.end(), tips.begin(), tips.end());
+        nn_tips_.stale = true;
+      }
+    }
+    if (eflags_.empty() || eflags_.size() > ne) {
+      precomputeEdgeVoxelCache();
+    } else if (eflags_.size() < ne) {
+      const size_t e0 = eflags_.size(), m = ne - e0;
+      std::vector<double> a(m * S), b(m * S);
+      for (size_t i = 0; i < m; i++) {
+        std::copy(states_[edges_[e0 + i].first].begin(), states_[edges_[e0 + i].first].end(), a.begin() + i * S);
+        std::copy(states_[edges_[e0 + i].second].begin(), states_[edges_[e0 + i].second].end(), b.begin() + i * S);
+      }
+      std::vector<uint32_t> fl(m);
+      std::shared_ptr<irt_setstore> scratch = scratch_store();
+      irt::check(ctx_, irt_voxelize_edges(ctx_, robot_.handle(), &space_, a.data(), b.data(), (int)S, (int64_t)m,
+                                          scratch.get(), fl.data(), nullptr, nullptr));
+      irt::check(ctx_, irt_setstore_append(ctx_, estore_, scratch.get(), 0, (int64_t)m, nullptr));
+      eflags_.insert(eflags_.end(), fl.begin(), fl.end());
+    }
+  }
   /// clear*VoxelCache (.cpp:1814-1829): drop the cached sets; validity words stay, like the reference's
   void clearVertexVoxelCache() { clear_store(vstore_); vflags_.clear(); tips_.clear(); nn_tips_.stale = true; }
   void clearEdgeVoxelCache() { clear_store(estore_); eflags_.clear(); }
@@ -1875,6 +1921,13 @@ private:
     auto it = adj_extra_.find(v);
     if (it != adj_extra_.end())
       for (auto &ne : it->second) fn(ne.first, ne.second);
+  }
+  /// an empty store on the environment's grid, destroyed with its last owner
+  std::shared_ptr<irt_setstore> scratch_store() {
+    irt_setstore *st = nullptr;
+    irt_grid g = env_voxels_.grid(venv_.inv_rotation);
+    irt::check(ctx_, irt_setstore_create(ctx_, &g, &st));
+    return std::shared_ptr<irt_setstore>(st, [](irt_setstore *x) { irt_setstore_destroy(x); });
   }
   void clear_store(irt_setstore *st) {
     const uint64_t off = 0;

@@ -450,6 +450,43 @@ class VoxelCachedLazyPRM:
         self.precomputeVertexVoxelCache()
         self.precomputeEdgeVoxelCache()
 
+    def extendVoxelCache(self):
+        """The batch form of the reference's compute-if-absent voxelizeVertex / voxelizeEdge (VoxelCachedLazyPRM.cpp:
+        2803-2837, 2879-2902) over the items the caches lack (_tail: vertices and edges that roadmapIk / addMilestone /
+        chainedPlan added since the caches were built): only they are voxelised, into scratch stores, and appended to
+        the cached stores, with their flags, edge info and tips.  A cache that does not exist yet is built whole.
+        Afterwards the next sweep is one K3 launch over every item.  Validity words are not touched."""
+        if self.world != 1:
+            raise NotImplementedError("extendVoxelCache runs on the full roadmap of one rank")
+        nv = len(self.states)
+        if not self._have_vcache or self.tips is None:
+            self.precomputeVertexVoxelCache()
+        elif len(self.vertex_flags) < nv:
+            v0 = len(self.vertex_flags)
+            scratch = SetStore(self.ctx, self.grid)
+            flags, tips = scratch.voxelize_vertices(self.robot, self.states[v0:])
+            self.vertex_store.append(scratch)
+            self._grow("vertex_flags", flags)
+            if len(self.tips) == v0:
+                self._grow("tips", tips)          # appended rows: the k-NN copy appends them too
+            elif not np.array_equal(self.tips[v0:nv].view(np.uint64), tips.view(np.uint64)):
+                self.tips = np.concatenate([self.tips[:v0], tips])
+                self._replaced("tips")
+        ne = len(self.edges)
+        if not self._have_ecache:
+            self.precomputeEdgeVoxelCache()
+        elif len(self.edge_flags) < ne:
+            e0 = len(self.edge_flags)
+            scratch = SetStore(self.ctx, self.grid)
+            # only the tail's endpoints: the FK of the whole roadmap would cost as much as the rebuild
+            ends, pairs = np.unique(self.edges[e0:], return_inverse=True)
+            info = scratch.voxelize_edges_indexed(self.robot, self.space, self.states[ends], pairs.reshape(-1, 2))
+            self.edge_store.append(scratch)
+            self._grow("edge_flags", info["flags"])
+            self.edge_info = dict(flags=self.edge_flags,
+                                  t_last=np.concatenate([self.edge_info["t_last"], info["t_last"]]),
+                                  nsamples=np.concatenate([self.edge_info["nsamples"], info["nsamples"]]))
+
     def clearVertexVoxelCache(self):
         """clearVertexVoxelCache (VoxelCachedLazyPRM.cpp:1814-1818): the cached sets go, validity words stay"""
         self.vertex_store = SetStore(self.ctx, self.grid)
