@@ -338,6 +338,42 @@ int irt_check_sets_dev(irt_ctx *ctx, const irt_setstore *store, const irt_env *e
  * size-independent checksum and for reporting. */
 int irt_check_sets_popcount(irt_ctx *ctx, const irt_setstore *store, const irt_env *env,
                             int64_t begin, int64_t end, uint64_t *stats);
+
+/* ---- incremental revalidation after an environment change (the replanning loop; the reference has no live-update
+ * API and re-checks every item) ----------------------------------------------------------------------------------
+ * A set's verdict can only change where one of its leaves overlaps a changed voxel: for a leaf with
+ * bits & (old ^ new) == 0, bits & new == bits & old.  The index lists, per leaf-block key, the sets with a leaf there
+ * and that leaf's bits, so a change re-checks only the sets whose leaves overlap it.
+ *
+ * Inverted index of a set store: for every leaf-block key, the (set index, leaf bits) of every set that has a leaf
+ * there.  Covers sets [0, irt_setindex_num_sets(ix)) of the store as it was when built; ~12 B per leaf + 8 B per key.
+ * IRT_ERR_CAPACITY when the store holds 2^32 sets or more.  The index belongs to its store and is built on the
+ * device (synchronous); it holds no pointer into the store's arrays, which appends may move. */
+typedef struct irt_setindex irt_setindex;
+int irt_setindex_create(irt_ctx *ctx, const irt_setstore *store, irt_setindex **out);
+void irt_setindex_destroy(irt_setindex *ix);
+int64_t irt_setindex_num_sets(const irt_setindex *ix);
+
+/* verdict_words (host, (end-begin+31)/32 words): on entry the words irt_check_sets(store, env_old, begin, end) gave,
+ * on return the words irt_check_sets(store, env_new, begin, end) gives, bit for bit.  flipped (host, may be NULL):
+ * the absolute indices of the sets whose bit changed, ascending; *n_flipped (may be NULL) their number.  stats (may
+ * be NULL): [0] changed leaf blocks, [1] sets re-checked, [2] 1 if the call swept the whole range instead.
+ * Synchronous.
+ *   Tail sets: sets in [irt_setindex_num_sets(ix), end) were appended after the build (irt_setstore_append, which
+ *     never changes existing sets); they are re-checked in full whenever a block changed.
+ *   The path is chosen from the input: when the index lists of the changed blocks hold more entries than a fixed
+ *     fraction of the range's leaves, the call sweeps the range with K3 instead (same words, same flips).
+ *   IRT_ERR_INVALID_ARGUMENT: NULL handles; env_old / env_new grids that differ (Ng, lim, inv_rot); a store whose Ng
+ *     differs from the environments'; begin < 0, end < begin or end > irt_setstore_num_sets(store); an index of
+ *     another store, or a stale one (the store's content was replaced by irt_setstore_import or irt_voxelize_*
+ *     after the build: rebuild the index); cap_flipped < 0; verdict_words NULL for a non-empty range.
+ *   IRT_ERR_CAPACITY: flipped != NULL and more than cap_flipped sets flipped; *n_flipped is set to the number needed.
+ *   Every argument is checked before anything runs; on any error verdict_words is unchanged.
+ *   env_old == env_new, or two equal grids, is a no-op with no flips. */
+int irt_check_sets_changed(irt_ctx *ctx, const irt_setstore *store, const irt_setindex *ix,
+                           const irt_env *env_old, const irt_env *env_new, int64_t begin, int64_t end,
+                           uint32_t *verdict_words, int64_t *flipped, int64_t cap_flipped, int64_t *n_flipped,
+                           int64_t *stats);
 /* ---- multi-GPU: verdict all-gather fused into K3 over peer memory (NVLink / NVSwitch) -----------
  * One process per GPU.  Every rank creates an exchange buffer, publishes its handle (host-side
  * all-gather of irt_xchg_handle_size() bytes, e.g. with torch.distributed / MPI) and connects.  A

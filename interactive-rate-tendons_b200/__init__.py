@@ -117,6 +117,7 @@ ABI_SYMBOLS = [
     "irt_valid_segment_count",
     "irt_check_sets", "irt_check_sets_dev", "irt_check_sets_popcount",
     "irt_check_sets_algorithmic_bytes",
+    "irt_setindex_create", "irt_setindex_destroy", "irt_setindex_num_sets", "irt_check_sets_changed",
     "irt_xchg_create", "irt_xchg_destroy", "irt_xchg_handle_size", "irt_xchg_export", "irt_xchg_connect",
     "irt_check_sets_allgather_dev", "irt_xchg_status",
     "irt_rmp_read", "irt_rmp_write", "irt_rmp_free",
@@ -191,6 +192,10 @@ def lib():
         "irt_check_sets_dev": (i32, [vp, vp, vp, i64, i64, vp, vp]),
         "irt_check_sets_popcount": (i32, [vp, vp, vp, i64, i64, vp]),
         "irt_check_sets_algorithmic_bytes": (i64, [vp, i64, i64]),
+        "irt_setindex_create": (i32, [vp, vp, C.POINTER(vp)]),
+        "irt_setindex_destroy": (None, [vp]),
+        "irt_setindex_num_sets": (i64, [vp]),
+        "irt_check_sets_changed": (i32, [vp, vp, vp, vp, vp, i64, i64, vp, vp, i64, vp, vp]),
         "irt_xchg_create": (i32, [vp, i32, i32, i64, C.POINTER(vp)]),
         "irt_xchg_destroy": (None, [vp]),
         "irt_xchg_handle_size": (i32, []),
@@ -660,6 +665,56 @@ class SetStore:
     def algorithmic_bytes(self, begin=0, end=None):
         end = self.num_sets if end is None else end
         return int(self.ctx.L.irt_check_sets_algorithmic_bytes(self.h, begin, end))
+
+    def check_changed(self, index, env_old, env_new, words, begin=0, end=None):
+        """Revalidation after an environment change (irt_check_sets_changed): `words` (uint32, the packed verdicts
+        check(env_old, begin, end) gave) become the words of check(env_new, begin, end), in place when they are a
+        contiguous uint32 array.  Only the sets whose leaves overlap the changed voxels, and the sets appended after
+        `index` was built, are re-checked.  Returns (words, flipped: int64 indices of the sets whose verdict changed,
+        ascending; stats: [changed leaf blocks, sets re-checked, 1 if the whole range was swept instead])."""
+        end = self.num_sets if end is None else end
+        words = _np(words, np.uint32)
+        if len(words) < (max(end - begin, 0) + 31) // 32:
+            raise IrtError(IRT_ERR_INVALID_ARGUMENT, "words must hold (end - begin + 31) // 32 entries")
+        stats = np.zeros(3, dtype=np.int64)
+        n_flipped = C.c_int64(0)
+        flipped = np.zeros(1024, dtype=np.int64)
+        for attempt in range(2):      # a change that flips more sets than the buffer holds: grow it, try once more
+            rc = self.ctx.L.irt_check_sets_changed(self.ctx.h, self.h, index.h, env_old.h, env_new.h, begin, end,
+                                                   _ptr(words), _ptr(flipped), len(flipped), C.byref(n_flipped),
+                                                   _ptr(stats))
+            if rc != IRT_ERR_CAPACITY or attempt == 1 or n_flipped.value <= len(flipped):
+                break
+            flipped = np.zeros(n_flipped.value, dtype=np.int64)
+        self.ctx.check(rc)
+        return words, flipped[:n_flipped.value].copy(), stats
+
+
+class SetIndex:
+    """Inverted index of a SetStore (irt_setindex): per leaf-block key, the sets with a leaf there and that leaf's
+    bits.  It covers the store's sets as they are when it is built; sets appended later are its tail, and replacing
+    the store's content makes it stale (SetStore.check_changed then raises)."""
+
+    def __init__(self, ctx, store):
+        self.ctx, self.store = ctx, store
+        h = C.c_void_p()
+        ctx.check(ctx.L.irt_setindex_create(ctx.h, store.h, C.byref(h)))
+        self.h = h
+
+    def close(self):
+        if getattr(self, "h", None) and getattr(self.ctx, "h", None):
+            self.ctx.L.irt_setindex_destroy(self.h)
+        self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @property
+    def num_sets(self):
+        return int(self.ctx.L.irt_setindex_num_sets(self.h))
 
 
 def state_metric(spec):

@@ -102,7 +102,20 @@ struct irt_setstore {
   uint32_t *d_keys = nullptr;     // [n_blocks]
   uint64_t *d_bits = nullptr;     // [n_blocks]
   size_t cap_sets = 0, cap_blocks = 0;
+  // bumped whenever the content is replaced (import, irt_voxelize_*), not by an append: an irt_setindex built at
+  // another generation describes sets that are no longer there
+  uint64_t generation = 0;
 };
+
+// Ng, limits and rotation all equal: voxel sets and grids of the two are comparable block by block
+inline bool same_grid(const irt_grid &a, const irt_grid &b) {
+  if (a.Ng != b.Ng) return false;
+  for (int i = 0; i < 6; i++)
+    if (a.lim[i] != b.lim[i]) return false;
+  for (int i = 0; i < 9; i++)
+    if (a.inv_rot[i] != b.inv_rot[i]) return false;
+  return true;
+}
 
 int irt_fail(irt_ctx *ctx, int status, const char *fmt, ...);
 GridDev make_grid_dev(const irt_grid &g);
@@ -132,6 +145,9 @@ int env_rebuild_occ(irt_ctx *ctx, irt_env *env, cudaStream_t st);
 int setstore_reserve(irt_ctx *ctx, irt_setstore *s, int64_t n_sets, int64_t n_blocks);
 int setstore_finalize(irt_ctx *ctx, irt_setstore *s, int64_t n_sets, int64_t n_blocks,
                       cudaStream_t st);
+// K3 over sets [begin, end) into device words, stream-ordered; the same argument checks as irt_check_sets_dev
+int check_sets_launch(irt_ctx *ctx, const irt_setstore *store, const irt_env *env, int64_t begin, int64_t end,
+                      uint32_t *d_verdict, cudaStream_t st);
 // d_row_off == nullptr: dense outputs p/R/t[n][cap_pts]; else packed rows, configuration i at row d_row_off[i].
 // d_range != nullptr: the batch is rows [lo, hi) of d_states and of the outputs, {lo, hi} read from device memory
 // when the kernels run (n = upper bound of hi - lo); work = fk_work_bytes(rb, n) bytes of device scratch private

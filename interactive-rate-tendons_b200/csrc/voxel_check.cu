@@ -456,8 +456,9 @@ append_gather_kernel(const uint64_t *__restrict__ src_off, const uint32_t *__res
 
 }  // namespace
 
-// used by voxel_raster.cu after it has filled the store on the device
+// the start of every replacement of a store's content (import, and voxel_raster.cu before it fills the store)
 int setstore_reserve(irt_ctx *ctx, irt_setstore *s, int64_t n_sets, int64_t n_blocks) {
+  s->generation++;
   return ensure_store_capacity(ctx, s, n_sets, n_blocks);
 }
 
@@ -664,7 +665,7 @@ int irt_setstore_import(irt_ctx *ctx, irt_setstore *s, int64_t n_sets, const uin
   for (int64_t i = 0; i < nb; i++)
     if (keys[i] >= nkeys) return irt_fail(ctx, IRT_ERR_OUT_OF_RANGE, "block key outside the grid");
   IRT_CUDA(ctx, cudaSetDevice(ctx->device));
-  int rc = ensure_store_capacity(ctx, s, n_sets, nb);
+  int rc = setstore_reserve(ctx, s, n_sets, nb);
   if (rc) return rc;
   cudaStream_t st = ctx->stream;
   IRT_CUDA(ctx, cudaMemcpyAsync(s->d_offsets, offsets, (size_t)(n_sets + 1) * 8, cudaMemcpyHostToDevice, st));
@@ -704,15 +705,6 @@ int irt_setstore_device_ptrs(const irt_setstore *s, const uint64_t **d_offsets,
   if (d_keys) *d_keys = s->d_keys;
   if (d_bits) *d_bits = s->d_bits;
   return IRT_OK;
-}
-
-static bool same_grid(const irt_grid &a, const irt_grid &b) {
-  if (a.Ng != b.Ng) return false;
-  for (int i = 0; i < 6; i++)
-    if (a.lim[i] != b.lim[i]) return false;
-  for (int i = 0; i < 9; i++)
-    if (a.inv_rot[i] != b.inv_rot[i]) return false;
-  return true;
 }
 
 // count + scan (one CUB scan of (leaves, sets) pairs), one read-back of the totals to size the growth, then the
@@ -854,6 +846,13 @@ static int check_sets_impl(irt_ctx *ctx, const irt_setstore *store, const irt_en
   IRT_CUDA(ctx, cudaGetLastError());
   return IRT_OK;
 }
+
+}  // extern "C"
+int check_sets_launch(irt_ctx *ctx, const irt_setstore *store, const irt_env *env, int64_t begin, int64_t end,
+                      uint32_t *d_verdict, cudaStream_t st) {
+  return check_sets_impl(ctx, store, env, begin, end, d_verdict, nullptr, st);
+}
+extern "C" {
 
 // ---- verdict exchange over peer memory (multi-GPU) ----------------------------------------------
 struct irt_xchg {

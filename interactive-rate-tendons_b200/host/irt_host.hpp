@@ -45,9 +45,10 @@
 #include "../../include/irt_b200.h"
 #ifdef IRT_TEST_OVER_STANDIN
 // built over the test-only stand-in of the C ABI (no GPU): irt_nnset_* come from a sequential host implementation,
-// irt_setstore_append from the stand-in's export / import
+// irt_setstore_append from the stand-in's export / import, irt_check_sets_changed from export + host comparison
 #include "../../tests/cpp/knn_standin.hpp"
 #include "../../tests/cpp/setstore_append_standin.hpp"
+#include "../../tests/cpp/env_delta_standin.hpp"
 #endif
 
 namespace irt {
@@ -1017,7 +1018,8 @@ public:
     irt::check(ctx_, irt_nnset_create(ctx_, 3, &tm, &nn_tips_.set));
   }
   ~VoxelCachedLazyPRM() {
-    irt_setstore_destroy(vstore_); irt_setstore_destroy(estore_); irt_env_destroy(env_);
+    irt_setindex_destroy(vindex_); irt_setindex_destroy(eindex_);
+    irt_setstore_destroy(vstore_); irt_setstore_destroy(estore_); irt_env_destroy(env_); irt_env_destroy(env_next_);
     irt_nnset_destroy(nn_states_.set); irt_nnset_destroy(nn_tips_.set);
   }
   void setRoadmap(std::vector<std::vector<double>> states, std::vector<std::pair<size_t, size_t>> edges) {
@@ -1196,6 +1198,7 @@ public:
     for (size_t i = 0; i < n; i++) std::copy(states_[i].begin(), states_[i].end(), flat.begin() + i * S);
     vflags_.assign(n, 0); tips_.assign(3 * n, 0.0);
     nn_tips_.stale = true;
+    vcache_builds_++;
     irt::check(ctx_, irt_voxelize_vertices(ctx_, robot_.handle(), flat.data(), (int)S, (int64_t)n, vstore_,
                                            vflags_.data(), tips_.data()));
   }
@@ -1207,6 +1210,7 @@ public:
       std::copy(states_[edges_[i].second].begin(), states_[edges_[i].second].end(), b.begin() + i * S);
     }
     eflags_.assign(n, 0);
+    ecache_builds_++;
     irt::check(ctx_, irt_voxelize_edges(ctx_, robot_.handle(), &space_, a.data(), b.data(), (int)S, (int64_t)n,
                                         estore_, eflags_.data(), nullptr, nullptr));
   }
@@ -1256,8 +1260,11 @@ public:
     }
   }
   /// clear*VoxelCache (.cpp:1814-1829): drop the cached sets; validity words stay, like the reference's
-  void clearVertexVoxelCache() { clear_store(vstore_); vflags_.clear(); tips_.clear(); nn_tips_.stale = true; }
-  void clearEdgeVoxelCache() { clear_store(estore_); eflags_.clear(); }
+  void clearVertexVoxelCache() {
+    clear_store(vstore_); vflags_.clear(); tips_.clear(); nn_tips_.stale = true;
+    irt_setindex_destroy(vindex_); vindex_ = nullptr;
+  }
+  void clearEdgeVoxelCache() { clear_store(estore_); eflags_.clear(); irt_setindex_destroy(eindex_); eindex_ = nullptr; }
   void clearVoxelCache() { clearVertexVoxelCache(); clearEdgeVoxelCache(); }
   size_t vertexVoxelCacheSize() const { return (size_t)irt_setstore_num_sets(vstore_); }
   size_t edgeVoxelCacheSize() const { return (size_t)irt_setstore_num_sets(estore_); }
@@ -1269,8 +1276,7 @@ public:
     if (vflags_.size() != states_.size() &&
         (vflags_.empty() || vflags_.size() > states_.size() || states_.size() - vflags_.size() > max_uncached_))
       precomputeVertexVoxelCache();
-    sweep(vstore_, vflags_, IRT_FLAG_NONCONVERGED | IRT_FLAG_LENGTH_LIMIT | IRT_FLAG_SELF_COLLISION | IRT_FLAG_BAD_STATE,
-          vertex_validity_);
+    sweep(vstore_, vflags_, kVertexInvalid, vertex_validity_, vwords_, vwords_n_);
     if (vertex_validity_.size() < states_.size()) {
       std::vector<size_t> ids;
       for (size_t v = vertex_validity_.size(); v < states_.size(); v++) ids.push_back(v);
@@ -1284,7 +1290,7 @@ public:
     if (eflags_.size() != edges_.size() &&
         (eflags_.empty() || eflags_.size() > edges_.size() || edges_.size() - eflags_.size() > max_uncached_))
       precomputeEdgeVoxelCache();
-    sweep(estore_, eflags_, IRT_FLAG_PARTIAL, edge_validity_);
+    sweep(estore_, eflags_, IRT_FLAG_PARTIAL, edge_validity_, ewords_, ewords_n_);
     if (edge_validity_.size() < edges_.size()) {
       std::vector<size_t> ids;
       for (size_t e = edge_validity_.size(); e < edges_.size(); e++) ids.push_back(e);
@@ -1406,6 +1412,30 @@ public:
     env_voxels_ = env_voxels;
     env_voxels_.upload_env(ctx_, env_);
     clearValidity();
+  }
+  /// the items whose VALIDITY_TRUE bit an updateEnvironment flipped, ascending
+  struct EnvironmentChange { std::vector<size_t> vertices, edges; };
+  /// Environment replacement that keeps what the change cannot reach.  A validity table that is current (a sweep
+  /// ran since the last clearValidity) is patched in place: only the cached sets whose leaves overlap the changed
+  /// voxels are re-checked on the device (irt_check_sets_changed over an inverted index of the cache, built on first
+  /// use), the items without a cached set in one scratch batch; items still unchecked since the sweep stay unchecked
+  /// and their lazy check uses the new grid.  A table that is not current is reset to VALIDITY_UNKNOWN, as
+  /// setEnvironment resets it.  Every look-up then answers what it would after setEnvironment(env_voxels); no sweep
+  /// is counted.  A chained plan keeps its path when none of the path's items flipped.
+  EnvironmentChange updateEnvironment(const collision::VoxelOctree &env_voxels) {
+    if (!env_next_) {
+      irt_grid g = env_voxels_.grid(venv_.inv_rotation);
+      irt::check(ctx_, irt_env_create(ctx_, &g, &env_next_));
+    }
+    env_voxels_ = env_voxels;
+    env_voxels_.upload_env(ctx_, env_next_);
+    irt_env *old = env_;
+    env_ = env_next_;   // everything that reads env_ sees the new grid
+    env_next_ = old;
+    EnvironmentChange ch;
+    ch.vertices = patchTable(true, old);
+    ch.edges = patchTable(false, old);
+    return ch;
   }
   const std::vector<unsigned> &vertexValidity() const { return vertex_validity_; }
   const std::vector<unsigned> &edgeValidity() const { return edge_validity_; }
@@ -1999,9 +2029,79 @@ private:
     for (size_t i = 0; i < k && d[i].first <= bound; i++) out.push_back(d[i].second);
     return out;
   }
-  void sweep(irt_setstore *st, const std::vector<uint32_t> &flags, uint32_t mask, std::vector<unsigned> &validity) {
+  /// updateEnvironment for the vertex (vert) or edge table: the items whose validity bit flipped, ascending
+  std::vector<size_t> patchTable(bool vert, irt_env *env_old) {
+    std::vector<unsigned> &table = vert ? vertex_validity_ : edge_validity_;
+    std::set<size_t> &unchecked = vert ? vertex_unchecked_ : edge_unchecked_;
+    const size_t n_items = vert ? states_.size() : edges_.size();
+    std::vector<size_t> flipped;
+    if (!(vert ? vertex_swept_ : edge_swept_)) {
+      table.assign(n_items, VALIDITY_UNKNOWN);
+      unchecked.clear();
+      return flipped;
+    }
+    std::vector<uint32_t> &words = vert ? vwords_ : ewords_;
+    const size_t n = vert ? vwords_n_ : ewords_n_;
+    if (n > 0) {
+      irt_setstore *st = vert ? vstore_ : estore_;
+      if ((size_t)irt_setstore_num_sets(st) < n) {   // the cache was cleared since the sweep: the same sets again
+        if (vert) precomputeVertexVoxelCache(); else precomputeEdgeVoxelCache();
+      }
+      const std::vector<uint32_t> &flags = vert ? vflags_ : eflags_;
+      const uint32_t mask = vert ? kVertexInvalid : IRT_FLAG_PARTIAL;
+      irt_setindex *ix = setIndex(vert, n);
+      std::vector<int64_t> hits(1024);
+      int64_t nh = 0;
+      int rc = irt_check_sets_changed(ctx_, st, ix, env_old, env_, 0, (int64_t)n, words.data(), hits.data(),
+                                      (int64_t)hits.size(), &nh, nullptr);
+      if (rc == IRT_ERR_CAPACITY) {   // more flips than the buffer holds: words are unchanged, try once more
+        hits.resize((size_t)nh);
+        rc = irt_check_sets_changed(ctx_, st, ix, env_old, env_, 0, (int64_t)n, words.data(), hits.data(),
+                                    (int64_t)hits.size(), &nh, nullptr);
+      }
+      irt::check(ctx_, rc);
+      for (int64_t k = 0; k < nh; k++) {
+        const size_t i = (size_t)hits[(size_t)k];
+        const bool hit = (words[i >> 5] >> (i & 31)) & 1u;
+        const unsigned v = (!hit && !(flags[i] & mask)) ? VALIDITY_TRUE : VALIDITY_UNKNOWN;
+        if ((table[i] & VALIDITY_TRUE) != v) flipped.push_back(i);
+        table[i] = v;
+      }
+    }
+    // items without a cached set when the table was swept, or added since with a known verdict: one scratch batch
+    std::vector<size_t> ids;
+    for (size_t i = n; i < n_items; i++)
+      if (!unchecked.count(i)) ids.push_back(i);
+    if (!ids.empty()) {
+      const std::vector<unsigned> now = vert ? checkVerticesNow(ids) : checkEdgesNow(ids);
+      for (size_t k = 0; k < ids.size(); k++) {
+        if ((table[ids[k]] & VALIDITY_TRUE) != (now[k] & VALIDITY_TRUE)) flipped.push_back(ids[k]);
+        table[ids[k]] = now[k];
+      }
+    }
+    std::sort(flipped.begin(), flipped.end());
+    return flipped;
+  }
+  /// the inverted index of the vertex or edge cache covering its first n sets, or all but at most maxUncached() of
+  /// them: built on first use, rebuilt when the cache was rebuilt since, or when its unindexed tail grew too long
+  irt_setindex *setIndex(bool vert, size_t n) {
+    irt_setindex *&ix = vert ? vindex_ : eindex_;
+    size_t &built = vert ? vindex_build_ : eindex_build_;
+    const size_t builds = vert ? vcache_builds_ : ecache_builds_;
+    if (!ix || built != builds || (int64_t)n - irt_setindex_num_sets(ix) > (int64_t)max_uncached_) {
+      irt_setindex_destroy(ix);
+      ix = nullptr;
+      irt::check(ctx_, irt_setindex_create(ctx_, vert ? vstore_ : estore_, &ix));
+      built = builds;
+    }
+    return ix;
+  }
+  /// K3 over every cached set; the verdict words and the number of sets they cover are kept for updateEnvironment
+  void sweep(irt_setstore *st, const std::vector<uint32_t> &flags, uint32_t mask, std::vector<unsigned> &validity,
+             std::vector<uint32_t> &words, size_t &covered) {
     const int64_t n = irt_setstore_num_sets(st);
-    std::vector<uint32_t> words((n + 31) / 32 + 1, 0);
+    words.assign((n + 31) / 32 + 1, 0);
+    covered = (size_t)n;
     if (n > 0) irt::check(ctx_, irt_check_sets(ctx_, st, env_, 0, n, words.data()));
     validity.assign(n, VALIDITY_UNKNOWN);
     for (int64_t i = 0; i < n; i++) {
@@ -2016,6 +2116,15 @@ private:
   irt_ctx *ctx_ = nullptr;
   irt_setstore *vstore_ = nullptr, *estore_ = nullptr;
   irt_env *env_ = nullptr;
+  irt_env *env_next_ = nullptr;   // updateEnvironment uploads the next grid here, then swaps it with env_
+  static constexpr uint32_t kVertexInvalid =
+      IRT_FLAG_NONCONVERGED | IRT_FLAG_LENGTH_LIMIT | IRT_FLAG_SELF_COLLISION | IRT_FLAG_BAD_STATE;
+  // the verdict words of the last sweep of each table and the sets they cover; the caches' inverted indices with the
+  // cache build they were made from
+  std::vector<uint32_t> vwords_, ewords_;
+  size_t vwords_n_ = 0, ewords_n_ = 0;
+  irt_setindex *vindex_ = nullptr, *eindex_ = nullptr;
+  size_t vcache_builds_ = 0, ecache_builds_ = 0, vindex_build_ = 0, eindex_build_ = 0;
   std::vector<std::vector<double>> states_;
   std::vector<std::pair<size_t, size_t>> edges_;
   std::vector<uint32_t> vflags_, eflags_;

@@ -24,8 +24,8 @@ torch.distributed (NCCL) only publishes the IPC handles once.  The plain all_gat
 """
 import numpy as np
 
-from . import (INVALID_MASK, FLAG_PARTIAL, KNN_MAX_K, Context, Env, NearestSet, SetStore, make_space, shard_range,
-               state_metric, tip_metric, unpack_verdicts)
+from . import (INVALID_MASK, FLAG_PARTIAL, KNN_MAX_K, Context, Env, NearestSet, SetIndex, SetStore, make_space,
+               shard_range, state_metric, tip_metric, unpack_verdicts)
 
 VALIDITY_UNKNOWN = 0  # VoxelCachedLazyPRM.h:598-601
 VALIDITY_TRUE = 1
@@ -206,6 +206,12 @@ class VoxelCachedLazyPRM:
         self._vertex_unchecked, self._edge_unchecked = set(), set()
         self.max_uncached = 4096     # more items than this without a cached set: the next sweep rebuilds the cache
         self._flag_tables = {}
+        # updateEnvironment: the verdict words of the last sweep of each table, (words, sets they cover); the grid the
+        # next environment is uploaded into; per cache, (SetIndex, store, cache build) of its inverted index
+        self._vertex_words = self._edge_words = self._swept_words = None
+        self._env_next = None
+        self._index = {"vertex": None, "edge": None}
+        self._cache_builds = {"vertex": 0, "edge": 0}
         # device copies of self.states / self.tips for the k-NN queries: [set, rows it holds, must be rebuilt]
         self._nn = None
         if isinstance(ctx, Context):
@@ -435,6 +441,7 @@ class VoxelCachedLazyPRM:
         self.vertex_flags, self.tips = self.vertex_store.voxelize_vertices(self.robot, self.states[lo:hi])
         self._replaced("tips")
         self._have_vcache = True
+        self._cache_builds["vertex"] += 1
         return self.vertex_flags
 
     def precomputeEdgeVoxelCache(self):
@@ -444,6 +451,7 @@ class VoxelCachedLazyPRM:
         self.edge_flags = info["flags"]
         self.edge_info = info
         self._have_ecache = True
+        self._cache_builds["edge"] += 1
         return info
 
     def precomputeVoxelCache(self):
@@ -490,6 +498,7 @@ class VoxelCachedLazyPRM:
     def clearVertexVoxelCache(self):
         """clearVertexVoxelCache (VoxelCachedLazyPRM.cpp:1814-1818): the cached sets go, validity words stay"""
         self.vertex_store = SetStore(self.ctx, self.grid)
+        self._index["vertex"] = None
         self.vertex_flags = self.tips = None
         self._replaced("tips")
         self._have_vcache = False
@@ -498,6 +507,7 @@ class VoxelCachedLazyPRM:
     def clearEdgeVoxelCache(self):
         """clearEdgeVoxelCache (VoxelCachedLazyPRM.cpp:1820-1824)"""
         self.edge_store = SetStore(self.ctx, self.grid)
+        self._index["edge"] = None
         self.edge_flags = None
         self._have_ecache = False
         self._xchg = {k: v for k, v in self._xchg.items() if k[0] == id(self.vertex_store)}
@@ -514,10 +524,83 @@ class VoxelCachedLazyPRM:
         self.env.update(blocks)
         self.clearValidity()
 
+    def updateEnvironment(self, blocks):
+        """Replace the obstacle grid like setEnvironment, but keep what the change cannot reach.  A validity table that
+        is current (a sweep ran since the last clearValidity) is patched in place: only the cached sets whose leaves
+        overlap the changed voxels are re-checked on the device (SetStore.check_changed over an inverted index of the
+        cache), the items without a cached set are re-checked in one scratch batch, and items still unchecked since
+        the sweep stay unchecked (their lazy check uses the new grid).  A table that is not current is reset to
+        VALIDITY_UNKNOWN, as setEnvironment resets it.  Every look-up then answers what it would after
+        setEnvironment(blocks); no sweep is counted.  Returns {"vertices", "edges"}: the int64 indices, ascending, of
+        the items whose VALIDITY_TRUE bit flipped -- a chained plan keeps its path when none of the path's did."""
+        if self.world != 1:
+            raise NotImplementedError("updateEnvironment runs on the full roadmap of one rank")
+        if self._env_next is None:
+            self._env_next = Env(self.ctx, self.grid)
+        self._env_next.update(blocks)
+        old = self.env
+        self.env, self._env_next = self._env_next, old          # everything that reads self.env sees the new grid
+        return {"vertices": self._patch_table("vertex", old), "edges": self._patch_table("edge", old)}
+
+    def _patch_table(self, kind, env_old):
+        """updateEnvironment for the vertex or the edge table: the indices of the items whose validity bit flipped"""
+        vert = kind == "vertex"
+        name = "vertex_validity" if vert else "edge_validity"
+        n_items = len(self.states) if vert else len(self.edges)
+        none = np.zeros(0, dtype=np.int64)
+        if not (self._vertex_swept if vert else self._edge_swept):
+            setattr(self, name, np.zeros(n_items, dtype=np.uint8))
+            (self._vertex_unchecked if vert else self._edge_unchecked).clear()
+            return none
+        table = getattr(self, name)
+        words, n = self._vertex_words if vert else self._edge_words
+        flipped = [none]
+        if n > 0:
+            if vert and not self._have_vcache:     # cleared since the sweep: the same sets again
+                self.precomputeVertexVoxelCache()
+            elif not vert and not self._have_ecache:
+                self.precomputeEdgeVoxelCache()
+            store = self.vertex_store if vert else self.edge_store
+            words, hits, _ = store.check_changed(self._set_index(kind, n), env_old, self.env, words, 0, n)
+            if vert:
+                self._vertex_words = (words, n)
+            else:
+                self._edge_words = (words, n)
+            if len(hits):
+                flags = np.asarray(self.vertex_flags if vert else self.edge_flags)[hits]
+                now = (((words[hits >> 5] >> (hits & 31).astype(np.uint32)) & 1) == 0) & \
+                      ((flags & (INVALID_MASK if vert else FLAG_PARTIAL)) == 0)
+                new = now.astype(np.uint8) * np.uint8(VALIDITY_TRUE)
+                flipped.append(hits[(table[hits] & VALIDITY_TRUE) != new])
+                table[hits] = new
+        # items without a cached set when the table was swept, or added since with a known verdict: one scratch batch
+        unchecked = self._vertex_unchecked if vert else self._edge_unchecked
+        ids = np.arange(n, n_items, dtype=np.int64)
+        if unchecked:
+            ids = ids[~np.isin(ids, np.fromiter(unchecked, dtype=np.int64, count=len(unchecked)))]
+        if len(ids):
+            new = self._check_vertices_now(ids) if vert else self._check_edges_now(ids)
+            flipped.append(ids[(table[ids] & VALIDITY_TRUE) != new])
+            table[ids] = new
+        return np.sort(np.concatenate(flipped))
+
+    def _set_index(self, kind, n):
+        """the inverted index of the vertex or edge cache, covering its first n sets or all but at most max_uncached
+        of them: built on first use, rebuilt when the cache was rebuilt since, or its unindexed tail grew too long"""
+        store = self.vertex_store if kind == "vertex" else self.edge_store
+        ent = self._index[kind]
+        if ent is None or ent[1] is not store or ent[2] != self._cache_builds[kind] or \
+                n - ent[0].num_sets > self.max_uncached:
+            if ent is not None:
+                ent[0].close()
+            ent = self._index[kind] = (SetIndex(self.ctx, store), store, self._cache_builds[kind])
+        return ent[0]
+
     # ---- validity sweeps ------------------------------------------------------------------------
     def _sweep(self, store, n_total, flags):
         import torch
         if n_total == 0:        # a roadmap without edges (or vertices): nothing collides
+            self._swept_words = np.zeros(0, dtype=np.uint32)
             return np.zeros(0, dtype=bool)
         lo, hi = self.shard(n_total)
         w = shard_words(n_total, self.world)
@@ -545,7 +628,8 @@ class VoxelCachedLazyPRM:
             if not stream:  # legacy default stream: the library ran on its own stream
                 self.ctx.synchronize()
         allw = gather_verdict_words(words, self.dist)
-        collides = assemble_verdicts(allw.cpu().numpy().view(np.uint32), n_total, self.world)
+        self._swept_words = allw.cpu().numpy().view(np.uint32)   # kept for updateEnvironment
+        collides = assemble_verdicts(self._swept_words, n_total, self.world)
         return collides
 
     def precomputeVertexValidity(self):
@@ -554,7 +638,9 @@ class VoxelCachedLazyPRM:
         if not self._have_vcache or self._tail(self.vertex_flags, len(self.states)) > self.max_uncached:
             self.precomputeVertexVoxelCache()
         n = len(self.states) - self._tail(self.vertex_flags, len(self.states))   # the sets the store holds
+        self._swept_words = None
         collides = self._sweep(self.vertex_store, n, self.vertex_flags)
+        self._vertex_words = (self._swept_words, n)
         invalid = self._gather_flags(self.vertex_flags, n, INVALID_MASK)
         self.vertex_validity = _validity_table(collides, invalid)
         if n < len(self.states):     # vertices that joined since (roadmapIk / addMilestone): one small batch
@@ -569,7 +655,9 @@ class VoxelCachedLazyPRM:
         if not self._have_ecache or self._tail(self.edge_flags, len(self.edges)) > self.max_uncached:
             self.precomputeEdgeVoxelCache()
         n = len(self.edges) - self._tail(self.edge_flags, len(self.edges))
+        self._swept_words = None
         collides = self._sweep(self.edge_store, n, self.edge_flags)
+        self._edge_words = (self._swept_words, n)
         invalid = self._gather_flags(self.edge_flags, n, FLAG_PARTIAL)
         self.edge_validity = _validity_table(collides, invalid)
         if n < len(self.edges):
