@@ -13,6 +13,9 @@
 #include "../../include/irt_b200.h"
 
 #define IRT_CAP_PTS_MAX 512  // upper bound on backbone points per shape (L/dL + 2)
+// doubles per tendon in a row of the constant-memory routing table: rx, ry, rdx, rdy, rddx, rddy and the
+// state-independent products rx^2, ry^2, rx ry, |r|^2 (= rx^2 + ry^2) of the RK4 stage's accumulations
+#define IRT_CT_WIDTH 10
 
 struct irt_ctx {
   int device = 0;
@@ -72,6 +75,7 @@ struct irt_robot {
   int state_size = 0;
   int max_points = 0;
   double *d_table = nullptr;
+  double *d_ctab = nullptr;     // [n_table][N][IRT_CT_WIDTH]: source of the constant-memory copy
   double *d_head = nullptr;
   double *d_node_t = nullptr;
   std::vector<double> node_t;

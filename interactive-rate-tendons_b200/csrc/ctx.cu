@@ -336,6 +336,18 @@ int irt_robot_create(irt_ctx *ctx, const irt_robot_desc *desc, irt_robot **out) 
   for (int i = 0; i < K; i++) routing_host(*desc, rb->node_t[i], &table[(size_t)(2 * i) * N * 6]);
   for (int q = 1; q < K; q++)  // RK4 mid stage of the step node q -> node q-1
     routing_host(*desc, rb->node_t[q] + 0.5 * desc->dL, &table[(size_t)(2 * q - 1) * N * 6]);
+  // the wide rows of the constant-memory copy: each tendon's 6 values and the products of r (rounded on their own)
+  std::vector<double> ctab((size_t)d.n_table * N * IRT_CT_WIDTH);
+  for (size_t k = 0; k < (size_t)d.n_table * N; k++) {
+    const double *src = &table[6 * k];
+    double *dst = &ctab[IRT_CT_WIDTH * k];
+    for (int i = 0; i < 6; i++) dst[i] = src[i];
+    const double rxx = src[0] * src[0], ryy = src[1] * src[1];
+    dst[6] = rxx;
+    dst[7] = ryy;
+    dst[8] = src[0] * src[1];
+    dst[9] = rxx + ryy;
+  }
   // head (first gap) stages for s = 0: times 0, h0/2 [, h0, h0 + h1/2]
   std::vector<double> head((size_t)4 * N * 6, 0.0);
   {
@@ -361,7 +373,8 @@ int irt_robot_create(irt_ctx *ctx, const irt_robot_desc *desc, irt_robot **out) 
     if (cudaMalloc(dp, v.size() * sizeof(double)) != cudaSuccess) return false;
     return cudaMemcpy(*dp, v.data(), v.size() * sizeof(double), cudaMemcpyHostToDevice) == cudaSuccess;
   };
-  if (!upload(table, &rb->d_table) || !upload(head, &rb->d_head) || !upload(rb->node_t, &rb->d_node_t)) {
+  if (!upload(table, &rb->d_table) || !upload(ctab, &rb->d_ctab) || !upload(head, &rb->d_head) ||
+      !upload(rb->node_t, &rb->d_node_t)) {
     irt_robot_destroy(rb);
     return irt_fail(ctx, IRT_ERR_CUDA, "robot table upload failed: %s",
                     cudaGetErrorString(cudaGetLastError()));
@@ -377,6 +390,7 @@ void irt_robot_destroy(irt_robot *rb) {
   if (!rb) return;
   cudaSetDevice(rb->ctx->device);
   if (rb->d_table) cudaFree(rb->d_table);
+  if (rb->d_ctab) cudaFree(rb->d_ctab);
   if (rb->d_head) cudaFree(rb->d_head);
   if (rb->d_node_t) cudaFree(rb->d_node_t);
   delete rb;

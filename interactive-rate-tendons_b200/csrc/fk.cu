@@ -147,44 +147,66 @@ __device__ __forceinline__ void routing_eval_simple(const RobotDev &rb, const do
   }
 }
 
-// Where a stage reads its routing row from.  RtPtr: a pointer (the shared-memory table, or the per-thread rows of the
-// irregular first gap).  RtConst: a row of the copy of the table in CONSTANT memory, named by a warp-uniform index:
-// the values arrive through the uniform datapath (LDCU -> uniform registers) and enter the FP64 instructions as
-// uniform-register operands.  That matters because the FP64 pipe's issue rate is bounded by register-file reads:
-// a DFMA with three distinct register pairs costs 3 issue cycles instead of 2 (irt_measure_fp64_rate mode 2:
-// 0.68 of the DFMA peak), and every routing value that comes from a uniform register is one pair less -- and the 36
-// values of a row no longer occupy 72 registers of every thread.
-constexpr int FK_CT_DOUBLES = 7680;   // 60 KB of the 64 KB constant bank: 213 rows of a 6-tendon robot
+// Where a stage reads its routing row from.  RtPtr: a pointer to [NT][6] values (the shared-memory table, or the
+// per-thread rows of the irregular first gap); it forms the products of r itself.  RtConst: a row of the wide copy
+// of the table in CONSTANT memory ([NT][IRT_CT_WIDTH]: r, r', r'' and the products rx^2, ry^2, rx ry, |r|^2 that the
+// host tabulated), named by a warp-uniform index: the values arrive through the uniform datapath (LDCU -> uniform
+// registers) and enter the FP64 instructions as uniform-register operands.  That matters because the FP64 pipe's
+// issue rate is bounded by register-file reads: a DFMA with three distinct register pairs costs 3 issue cycles
+// instead of 2 (irt_measure_fp64_rate mode 2: 0.68 of the DFMA peak), and every routing value that comes from a
+// uniform register is one pair less -- and the values of a row occupy no registers of any thread.
+constexpr int FK_CT_DOUBLES = 8192;   // the whole 64 KB constant bank: 136 rows of a 6-tendon robot
 __constant__ double c_fk_tab[FK_CT_DOUBLES];
 struct RtPtr {
   const double *p;
-  __device__ __forceinline__ double operator[](int i) const { return p[i]; }
+  __device__ __forceinline__ double rx(int j) const { return p[6 * j + 0]; }
+  __device__ __forceinline__ double ry(int j) const { return p[6 * j + 1]; }
+  __device__ __forceinline__ double dx(int j) const { return p[6 * j + 2]; }
+  __device__ __forceinline__ double dy(int j) const { return p[6 * j + 3]; }
+  __device__ __forceinline__ double ddx(int j) const { return p[6 * j + 4]; }
+  __device__ __forceinline__ double ddy(int j) const { return p[6 * j + 5]; }
+  // rounded like the host's table (no contraction), so both paths see the same values
+  __device__ __forceinline__ double rxx(int j) const { return __dmul_rn(rx(j), rx(j)); }
+  __device__ __forceinline__ double ryy(int j) const { return __dmul_rn(ry(j), ry(j)); }
+  __device__ __forceinline__ double rxy(int j) const { return __dmul_rn(rx(j), ry(j)); }
+  __device__ __forceinline__ double rr(int j) const { return __dadd_rn(rxx(j), ryy(j)); }
 };
 struct RtConst {
   int base;
-  __device__ __forceinline__ double operator[](int i) const { return c_fk_tab[base + i]; }
+  __device__ __forceinline__ double at(int j, int k) const { return c_fk_tab[base + IRT_CT_WIDTH * j + k]; }
+  __device__ __forceinline__ double rx(int j) const { return at(j, 0); }
+  __device__ __forceinline__ double ry(int j) const { return at(j, 1); }
+  __device__ __forceinline__ double dx(int j) const { return at(j, 2); }
+  __device__ __forceinline__ double dy(int j) const { return at(j, 3); }
+  __device__ __forceinline__ double ddx(int j) const { return at(j, 4); }
+  __device__ __forceinline__ double ddy(int j) const { return at(j, 5); }
+  __device__ __forceinline__ double rxx(int j) const { return at(j, 6); }
+  __device__ __forceinline__ double ryy(int j) const { return at(j, 7); }
+  __device__ __forceinline__ double rxy(int j) const { return at(j, 8); }
+  __device__ __forceinline__ double rr(int j) const { return at(j, 9); }
 };
 
-// (v', u', sigma_i) at one RK4 stage.  rt: [NT][6] routing (RtPtr or RtConst).
+// (v', u', sigma_i) at one RK4 stage.  rt: the routing of the NT tendons (RtPtr or RtConst).
 template <int NT, typename RT>
 __device__ __forceinline__ void vu_dot(const RT &rt, const double (&tau)[NT],
                                        const double (&Kse)[3], const double (&Kbt)[3],
                                        const double (&v)[3], const double (&u)[3],
                                        double (&vd)[3], double (&ud)[3], double (&sig)[NT]) {
-  // symmetric A (00,01,02,11,12,22), full B (row-major), symmetric H, a, b
-  double a00 = 0, a01 = 0, a02 = 0, a11 = 0, a12 = 0, a22 = 0;
+  // symmetric A (00,01,02,11,12,22), full B (row-major), symmetric H, a, b.  The stiffness diagonals K_se, K_bt
+  // are the start values of the sums they belong to.
+  double a00 = 0, a01 = 0, a02 = -0.0, a11 = 0, a12 = -0.0, a22 = Kse[2];
   double b00 = 0, b01 = 0, b02 = 0, b10 = 0, b11 = 0, b12 = 0, b20 = 0, b21 = 0, b22 = 0;
-  double h00 = 0, h01 = 0, h02 = 0, h11 = 0, h12 = 0, h22 = 0;
+  double h00 = Kbt[0], h01 = 0, h02 = 0, h11 = Kbt[1], h12 = 0, h22 = Kbt[2];
   // sums that are built with plain additions start from -0.0: (-0.0) + x == x for every x, so the first tendon's
   // "0 + x" folds away (with +0.0 it may not: 0 + (-0) is +0), one FP64 instruction less per sum and stage; the
   // value of a sum can differ from the +0.0 start only in the sign of an exact zero
-  double av0 = -0.0, av1 = -0.0, av2 = -0.0, bv0 = 0, bv1 = 0, bv2 = -0.0;
-  double esum = -0.0, erx = -0.0, ery = -0.0, exx = 0, eyy = 0, exy = 0;
+  double av0 = -0.0, av1 = -0.0, av2 = -0.0, bv0 = 0, bv1 = 0, bv2 = 0;
+  double esum = -0.0;
 #pragma unroll
   for (int j = 0; j < NT; j++) {
-    const double rx = rt[6 * j + 0], ry = rt[6 * j + 1];
-    const double dx = rt[6 * j + 2], dy = rt[6 * j + 3];
-    const double ddx = rt[6 * j + 4], ddy = rt[6 * j + 5];
+    const double rx = rt.rx(j), ry = rt.ry(j);
+    const double dx = rt.dx(j), dy = rt.dy(j);
+    const double ddx = rt.ddx(j), ddy = rt.ddy(j);
     // q = u x r + r' + v        (r_z = r'_z = r''_z = 0)
     const double qx = fma(-u[2], ry, dx + v[0]);
     const double qy = fma(u[2], rx, dy + v[1]);
@@ -194,20 +216,27 @@ __device__ __forceinline__ void vu_dot(const RT &rt, const double (&tau)[NT],
     sig[j] = s2 * rs;
     const double e = tau[j] * rs;        // tau / sigma
     const double c3 = e * (rs * rs);     // tau / sigma^3
-    const double mx = ry * qz, my = -rx * qz, mz = fma(rx, qy, -ry * qx);  // m = r x q
-    const double cqx = c3 * qx, cqy = c3 * qy, cqz = c3 * qz;
-    const double cmx = c3 * mx, cmy = c3 * my, cmz = c3 * mz;
-    a00 = fma(-cqx, qx, a00); a01 = fma(-cqx, qy, a01); a02 = fma(-cqx, qz, a02);
-    a11 = fma(-cqy, qy, a11); a12 = fma(-cqy, qz, a12); a22 = fma(-cqz, qz, a22);
+    // With r_z = 0, m = r x q = (ry qz, -rx qz, mz), and t = c3 qz q, kap = e - c3 qz^2:
+    //   A_i = e I - c3 q q^T                 z row: -t (+ e on the diagonal: kap)
+    //   B_i = e r^ - c3 m q^T                rows 0, 1: -ry t, rx t (+ e r^: ry kap, -rx kap in column 2);
+    //                                        row 2: -c3 mz q (+ e r^: -e ry, e rx)
+    //   H_i = e (|r|^2 I - r r^T) - c3 m m^T  = kap [[ry^2, -rx ry], [-rx ry, rx^2]] in the top-left block,
+    //                                          -+ r (c3 qz mz) in column 2, e |r|^2 - c3 mz^2 on the diagonal
+    // so most accumulations are one register pair against a routing value or product that the fast path reads
+    // from a uniform register
+    const double mz = fma(rx, qy, -ry * qx);
+    const double cqx = c3 * qx, cqy = c3 * qy, cqz = c3 * qz, cmz = c3 * mz;
+    const double tx = cqz * qx, ty = cqz * qy, kap = fma(-cqz, qz, e), tzm = cqz * mz;
+    a00 = fma(-cqx, qx, a00); a01 = fma(-cqx, qy, a01); a11 = fma(-cqy, qy, a11);
+    a02 -= tx; a12 -= ty; a22 += kap;
     esum += e;
-    b00 = fma(-cmx, qx, b00); b01 = fma(-cmx, qy, b01); b02 = fma(-cmx, qz, b02);
-    b10 = fma(-cmy, qx, b10); b11 = fma(-cmy, qy, b11); b12 = fma(-cmy, qz, b12);
+    b00 = fma(-ry, tx, b00); b01 = fma(-ry, ty, b01); b02 = fma(ry, kap, b02);
+    b10 = fma(rx, tx, b10); b11 = fma(rx, ty, b11); b12 = fma(-rx, kap, b12);
     b20 = fma(-cmz, qx, b20); b21 = fma(-cmz, qy, b21); b22 = fma(-cmz, qz, b22);
-    const double erxj = e * rx, eryj = e * ry;
-    erx += erxj; ery += eryj;
-    h00 = fma(-cmx, mx, h00); h01 = fma(-cmx, my, h01); h02 = fma(-cmx, mz, h02);
-    h11 = fma(-cmy, my, h11); h12 = fma(-cmy, mz, h12); h22 = fma(-cmz, mz, h22);
-    exx = fma(erxj, rx, exx); eyy = fma(eryj, ry, eyy); exy = fma(erxj, ry, exy);
+    b20 = fma(-e, ry, b20); b21 = fma(e, rx, b21);
+    h00 = fma(kap, rt.ryy(j), h00); h01 = fma(-kap, rt.rxy(j), h01); h11 = fma(kap, rt.rxx(j), h11);
+    h02 = fma(-ry, tzm, h02); h12 = fma(rx, tzm, h12);
+    h22 = fma(e, rt.rr(j), h22); h22 = fma(-cmz, mz, h22);
     // w = u x (q + r') + r''
     const double gx = qx + dx, gy = qy + dy, gz = qz;
     const double wx = fma(u[1], gz, fma(-u[2], gy, ddx));
@@ -218,12 +247,10 @@ __device__ __forceinline__ void vu_dot(const RT &rt, const double (&tau)[NT],
     const double ax = fma(e, wx, -cqx * qw), ay = fma(e, wy, -cqy * qw), az = fma(e, wz, -cqz * qw);
     av0 += ax; av1 += ay; av2 += az;
     // b_i = r x a_i
-    bv0 = fma(ry, az, bv0); bv1 = fma(-rx, az, bv1); bv2 += fma(rx, ay, -ry * ax);
+    bv0 = fma(ry, az, bv0); bv1 = fma(-rx, az, bv1); bv2 = fma(rx, ay, bv2); bv2 = fma(-ry, ax, bv2);
   }
-  // A += (sum e) I + K_se ;  B += sum e r^ ;  H += sum e (|r|^2 I - r r^T) + K_bt
-  a00 += esum + Kse[0]; a11 += esum + Kse[1]; a22 += esum + Kse[2];
-  b02 += ery; b12 -= erx; b20 -= ery; b21 += erx;
-  h00 += eyy + Kbt[0]; h11 += exx + Kbt[1]; h22 += (exx + eyy) + Kbt[2]; h01 -= exy;
+  // A += (sum e) I on the diagonal entries whose sums do not hold it yet, and K_se
+  a00 += esum + Kse[0]; a11 += esum + Kse[1];
 
   // right-hand sides (tendon_deriv.cpp:159-161), K diagonal
   const double kv0 = Kse[0] * v[0], kv1 = Kse[1] * v[1], kv2 = Kse[2] * (v[2] - 1.0);
@@ -650,8 +677,9 @@ __global__ void __launch_bounds__(FK_THREADS, FK_BLOCKS_PER_SM) fk_rk4_fp64_kern
       // every lane of the warp takes the regular step q (the common case: buckets are warps of equal step
       // counts): the routing rows come from constant memory by a warp-uniform index, the step size is uniform
       if (a.use_const && __all_sync(0xffffffffu, integ && q <= K - 1)) {
-        const int b0 = 2 * q * NT * 6;
-        rk4_step<NT, RtConst>(x, tau, Kse, Kbt, rb.dL, RtConst{b0}, RtConst{b0 - NT * 6}, RtConst{b0 - 2 * NT * 6});
+        const int b0 = 2 * q * NT * IRT_CT_WIDTH;
+        rk4_step<NT, RtConst>(x, tau, Kse, Kbt, rb.dL, RtConst{b0}, RtConst{b0 - NT * IRT_CT_WIDTH},
+                              RtConst{b0 - 2 * NT * IRT_CT_WIDTH});
         emit_node<NT>(o, row_base, K - q + 1, rb.node_t[q - 1], x, rz);
         continue;
       }
@@ -917,12 +945,12 @@ int fk_launch(irt_ctx *ctx, const irt_robot *rb, const double *d_states, int64_t
   static std::mutex ct_mutex;
   static unsigned long long ct_owner[64] = {};
   std::unique_lock<std::mutex> ct_lock(ct_mutex, std::defer_lock);
-  const size_t tab_doubles = (size_t)d.n_table * d.n_tendons * 6;
+  const size_t tab_doubles = (size_t)d.n_table * d.n_tendons * IRT_CT_WIDTH;
   if (tab_doubles <= (size_t)FK_CT_DOUBLES && ctx->device >= 0 && ctx->device < 64) {
     ct_lock.lock();
     if (ct_owner[ctx->device] != rb->uid) {
       IRT_CUDA(ctx, cudaDeviceSynchronize());
-      IRT_CUDA(ctx, cudaMemcpyToSymbolAsync(c_fk_tab, rb->d_table, tab_doubles * sizeof(double), 0,
+      IRT_CUDA(ctx, cudaMemcpyToSymbolAsync(c_fk_tab, rb->d_ctab, tab_doubles * sizeof(double), 0,
                                             cudaMemcpyDeviceToDevice, st));
       IRT_CUDA(ctx, cudaStreamSynchronize(st));
       ct_owner[ctx->device] = rb->uid;
